@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 3 --warmup 3            # our arm (CUDA, through the C ABI)
     python bench.py --impl reference --gpus 1 --steps 1      # the reference's CPU path on the host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # one rank per GPU, weak scaling by image
+    python bench.py --steps 3 --dump-outputs bench_outputs   # + the last timed step's outputs as .npy files
 
 Workload = BASELINE.json configs[1]: "Global view: 64 synthetic 5000x5000 images downscaled to
 max_pixels=1280*28*28" -> per image 980x980, grid (1,70,70), 4900 patches, 1225 vision tokens.  One step =
@@ -17,6 +18,9 @@ zv_visual_forward (32-block tower + merger), random-init Qwen2.5-VL-3B vision we
             against the measured dense bf16 peak; `roofline_k1` / `roofline_attn` give the other kernel classes.
 `cpu_baseline`: the reference's own CPU path (Pillow + HF PIL processor + HF torch tower, fp32) on a bounded
             sample of the same workload, on this box's host cores.
+
+Inputs (weights, pixels) are generated from fixed seeds, so two builds run with the same arguments see the same inputs
+and their --dump-outputs directories can be compared file by file.
 """
 import argparse
 import ctypes as C
@@ -260,6 +264,22 @@ def config3_sharded(enc, visual, dev, rank, world, op_dtype, n_crops):
 
 
 # ------------------------------------------------------------------------------------------- our arm (CUDA)
+DUMP_ROWS = 4096            # 4096 x 2048 float32 = 32 MiB of embeddings
+
+
+def dump_outputs(out_dir, emb, grid, crop):
+    """What one step hands its caller, as .npy files: embeddings.npy (a fixed, seeded sample of DUMP_ROWS rows in
+    ascending order, all rows when there are fewer; float32 holds the fp16 / bf16 values exactly), image_grid_thw.npy
+    and crop_boxes.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = emb.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS else np.arange(n)
+    sample = emb[torch.from_numpy(rows).to(emb.device)].float().cpu().numpy()
+    np.save(os.path.join(out_dir, "embeddings.npy"), sample)
+    np.save(os.path.join(out_dir, "image_grid_thw.npy"), np.asarray(grid, np.float64))
+    np.save(os.path.join(out_dir, "crop_boxes.npy"), np.asarray(crop, np.float64))
+
+
 def run_ours(args):
     import torch.distributed as dist
     from zoomearth_b200 import FusedImageProcessor, FusedVisual, ZoomEncoder, _lib
@@ -313,17 +333,18 @@ def run_ours(args):
             pg, gather_kind = None, "nccl all_gather_into_tensor"
 
     def step():
+        """(embeddings of every rank, or None while the fused gather is in flight; grids; crop boxes)"""
         if pg is not None:
             pg.begin_step()                                # waits for the PREVIOUS step's cross-rank barrier, flips buffers
-            enc.encode(images, None, gather=pg, gather_row=rank * tokens_step)
+            _, grid, crop = enc.encode(images, None, gather=pg, gather_row=rank * tokens_step)
             pg.end_step()                                  # this step's barrier runs on a side stream behind the kernels
-            return None
-        emb, grid, _ = enc.encode(images, None)
+            return None, grid, crop
+        emb, grid, crop = enc.encode(images, None)
         if world > 1:
             out = torch.empty((world * emb.shape[0], emb.shape[1]), dtype=emb.dtype, device=dev)
             dist.all_gather_into_tensor(out, emb)          # C1: gather of the output embeddings (equal shards)
-            return out
-        return emb
+            return out, grid, crop
+        return emb, grid, crop
 
     def barrier():
         if pg is not None:
@@ -339,7 +360,7 @@ def run_ours(args):
     if world > 1:
         # correctness of the data path being timed: what step() leaves on every rank must be, bit for bit, NCCL's
         # all_gather_into_tensor of the per-rank embeddings (checked once, outside the timed region)
-        got = step()
+        got, _, _ = step()
         got = (pg.finish() if pg is not None else got).clone()
         barrier()
         emb, _, _ = enc.encode(images, None)
@@ -359,7 +380,7 @@ def run_ours(args):
     e0.record()
     launches = 0
     for _ in range(args.steps):
-        step()
+        last = step()
         launches += enc.last_launches
     if pg is not None:
         pg.finish()                                        # inside the timed region: every step's gather has landed
@@ -367,6 +388,11 @@ def run_ours(args):
     barrier()
     lib.zv_timing_enable(0)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        emb, grid, crop = last
+        dump_outputs(args.dump_outputs, emb if pg is None else pg.finish(), grid, crop)
+        del emb
+    del last
     ms = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -535,7 +561,13 @@ def main():
     ap.add_argument("--nccl-gather", action="store_true", help="gather embeddings with NCCL instead of the fused peer stores")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (rank 0; our arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
