@@ -25,8 +25,10 @@
  *                         rescale, normalize, patchify) as one fused device pass
  *   zv_plan_*             HF:models/qwen2_5_vl/modeling_qwen2_5_vl.py:382-409 (rot_pos_emb ids),
  *                         :411-451 (get_window_index), :470-496 (cu_window_seqlens, cu_seqlens)
- *   zv_weights_*          state-dict import of `visual.*` (HF:modeling_qwen2_5_vl.py:345-380 module tree)
- *   zv_visual_forward     HF:modeling_qwen2_5_vl.py:455-518 (Qwen2_5_VisionTransformerPretrainedModel.forward)
+ *   zv_weights_*          state-dict import of `visual.*` (HF:modeling_qwen2_5_vl.py:345-380 module tree; Qwen2-VL:
+ *                         HF:models/qwen2_vl/modeling_qwen2_vl.py VisionMlp / Qwen2VLVisionBlock / PatchMerger)
+ *   zv_visual_forward     HF:modeling_qwen2_5_vl.py:455-518 (Qwen2_5_VisionTransformerPretrainedModel.forward), or with
+ *                         tower_kind = ZV_TOWER_QWEN2 Qwen2VisionTransformerPretrainedModel.forward
  *   zv_visual_forward_into  + HF:modeling_qwen2_5_vl.py:1301-1307 (get_placeholder_mask + masked_scatter into
  *                         inputs_embeds; reference copy src/train/RL/.../open_r1/model/modeling_qwen2_vl.py:1191-1207)
  *   zv_rope_index         reference .../open_r1/model/modeling_qwen2_vl.py:967-1114 (get_rope_index; by flag the
@@ -58,6 +60,11 @@ typedef enum zv_err {
 
 enum { ZV_F32 = 0, ZV_BF16 = 1, ZV_F16 = 2 };   /* element types at the boundary */
 enum { ZV_ORDER_HF = 0, ZV_ORDER_WINDOW = 1 }; /* patch row order: HF merge-group raster, or tower window order */
+/* Vision tower family.  ZV_TOWER_QWEN25: Qwen2.5-VL (RMSNorm, SwiGLU, window attention, HF:modeling_qwen2_5_vl.py).
+ * ZV_TOWER_QWEN2: Qwen2-VL (LayerNorm with bias, fc1 -> QuickGELU -> fc2, full attention in every block,
+ * HF:models/qwen2_vl/modeling_qwen2_vl.py Qwen2VisionTransformerPretrainedModel); requires fullatt_mask_lo to cover all
+ * `depth` blocks and inter = 5120. */
+enum { ZV_TOWER_QWEN25 = 0, ZV_TOWER_QWEN2 = 1 };
 
 /* Processor + model constants (defaults = Qwen2.5-VL-3B vision config + OPENAI_CLIP statistics). */
 typedef struct zv_cfg {
@@ -80,6 +87,8 @@ typedef struct zv_cfg {
   float   std[3];
   float   eps;          /* 1e-6 */
   float   reserved_f;
+  int32_t tower_kind;   /* ZV_TOWER_QWEN25 (zv_default_cfg) or ZV_TOWER_QWEN2 */
+  int32_t reserved_i;
 } zv_cfg;
 
 ZV_API const char* zv_version(void);
@@ -224,8 +233,8 @@ ZV_API int64_t zv_last_launch_count(void);
 
 /* Optional per-kernel-class device timing (CUDA events on the launching stream around every launch of that
  * class).  Classes: 0 k1 hpass, 1 k1 vpass, 2 gemm store, 3 gemm qkv+rope, 4 gemm residual, 5 gemm swiglu,
- * 6 gemm gelu, 7 gemm scatter, 8 attention (window layers), 9 attention (full layers), 10 rmsnorm + cast_rows_ss,
- * 11 gather. */
+ * 6 gemm gelu, 7 gemm scatter, 8 attention (window layers), 9 attention (full layers), 10 rmsnorm / layernorm +
+ * cast_rows_ss / cast_rows_ln, 11 gather, 12 gemm quickgelu (Qwen2-VL fc1). */
 ZV_API void zv_timing_enable(int on);
 ZV_API void zv_timing_reset(void);
 ZV_API int zv_timing_read(int kernel_class, double* ms_total, int64_t* count);

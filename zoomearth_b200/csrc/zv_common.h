@@ -35,7 +35,7 @@ class NvtxRange {
 // Kernel classes for the optional event timing (zv_timing_*): one id per kernel template.
 enum KernelClass { KC_K1_HPASS = 0, KC_K1_VPASS = 1, KC_GEMM_STORE = 2, KC_GEMM_QKV = 3, KC_GEMM_RESID = 4,
                    KC_GEMM_SWIGLU = 5, KC_GEMM_GELU = 6, KC_GEMM_SCATTER = 7, KC_ATTN_WINDOW = 8, KC_ATTN_FULL = 9,
-                   KC_RMSNORM = 10, KC_GATHER = 11, KC_COUNT = 12 };
+                   KC_RMSNORM = 10, KC_GATHER = 11, KC_GEMM_QGELU = 12, KC_COUNT = 13 };
 // RAII: records an event pair around the launches issued in its scope when timing is enabled.
 class KernelTimer {
  public:

@@ -7,6 +7,10 @@
 //   EPI_SWIGLU   silu(gate+bg) * (up+bu) -> bf16              mlp :88 (gate/up rows interleaved per 128)
 //   EPI_GELU     gelu_erf(acc + bias) -> bf16                 merger.mlp.0/1 :138-140
 //   EPI_SCATTER  (acc + bias) -> row scatter[row]             merger.mlp.2 + un-reorder :512-513
+// and, for the Qwen2-VL tower (HF models/qwen2_vl/modeling_qwen2_vl.py), the LayerNorm-fold variants
+//   EPI_QKV_ROPE_LN  r * (acc - mu * c) + b', then the rotary    norm1 + attn.qkv
+//   EPI_RESID_LN     EPI_RESID with per-slot (mean, M2) of the new rows   attn.proj / mlp.fc2 + residual
+//   EPI_QGELU        quick_gelu(r * (acc - mu * c) + b') -> 16-bit       norm2 + mlp.fc1 + QuickGELU
 //
 // Structure (one CTA per SM, 384 threads): warp 0 = TMA producer (one elected lane), warp 1 = MMA issuer
 // (one elected lane, tcgen05.mma M=128 x N=BN x K=16 from 128B-swizzled smem tiles), warp 2 = TMEM
@@ -42,6 +46,8 @@ constexpr int kXposeBytesPerWarp = 32 * kXposePitch * 4;
 // then one [32][88] 16-bit output tile per lane quarter
 constexpr int kQkvRope0 = 24 * 32 * 8, kQkvRope1 = 16 * 32 * 8, kQkvTilePitch = 88, kQkvTile = 32 * kQkvTilePitch * 2;
 constexpr int kQkvStageBytes = 4 * kQkvRope0 + 4 * kQkvRope1 + 4 * kQkvTile;
+__host__ __device__ constexpr bool is_resid(int e) { return e == EPI_RESID || e == EPI_RESID_LN; }
+__host__ __device__ constexpr bool is_qkv(int e) { return e == EPI_QKV_ROPE || e == EPI_QKV_ROPE_LN; }
 template <int BN, int CG, int EPI = 0> struct Cfg {
   static constexpr int kBRows = BN / CG;                       // B rows staged per CTA (half the tile in a CTA pair)
   static constexpr int kABytes = BM * BK * 2;
@@ -50,13 +56,14 @@ template <int BN, int CG, int EPI = 0> struct Cfg {
   // the residual epilogue transposes its tile through shared memory (8 warps x 4.5 KB): one pipeline stage less
   // ... and the QKV epilogue keeps each row's rotary (cos, sin) pairs and a 32 x 80 output tile per lane quarter there
   // ... and the scatter epilogue regroups its 16-bit rows there so that four lanes store 64 contiguous bytes of a row
-  static constexpr int kXposeBytes = (EPI == EPI_RESID || EPI == EPI_SCATTER) ? 8 * kXposeBytesPerWarp : EPI == EPI_QKV_ROPE ? kQkvStageBytes : 0;
-  static constexpr int kStages = ((kBRows > 128) ? 4 : 6) - ((EPI == EPI_RESID || EPI == EPI_QKV_ROPE || EPI == EPI_SCATTER) ? 1 : 0);
+  static constexpr int kXposeBytes = (is_resid(EPI) || EPI == EPI_SCATTER) ? 8 * kXposeBytesPerWarp : is_qkv(EPI) ? kQkvStageBytes : 0;
+  static constexpr int kStages = ((kBRows > 128) ? 4 : 6) - ((is_resid(EPI) || is_qkv(EPI) || EPI == EPI_SCATTER) ? 1 : 0);
   static constexpr int kBarBytes = 256;
   static constexpr int kSmemBytes = kStages * kStageBytes + kBarBytes + kXposeBytes + 1024;   // +1024: manual alignment slack
 };
 
 __device__ __forceinline__ float silu(float x) { return __fdividef(x, 1.0f + __expf(-x)); }
+__device__ __forceinline__ float quick_gelu(float x) { return __fdividef(x, 1.0f + __expf(-1.702f * x)); }
 __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f)); }
 // two fp32 -> packed 16-bit pair, bf16 or fp16 (warp-uniform choice)
 __device__ __forceinline__ uint32_t pack2(float a, float b, bool f16) {
@@ -86,6 +93,30 @@ __device__ __forceinline__ float row_rscale(const GemmArgs& g, int row, bool val
   return rsqrtf(s / (float)g.norm_dim + g.norm_eps);
 }
 
+// folded LayerNorm, consumer side: mean and 1 / std of accumulator row `row` from its producer's 20 slot statistics
+// (64 columns each), merged in slot order with Chan's formula - no E[x^2] - E[x]^2 cancellation (0 and 1 when unused)
+__device__ __forceinline__ void row_ln_stats(const GemmArgs& g, int row, bool valid, float& mu, float& rs) {
+  mu = 0.f; rs = 1.f;
+  if (!valid) return;
+  const float4* p = reinterpret_cast<const float4*>(g.row_ln + (int64_t)row * kSsParts);
+  float mean = 0.f, m2 = 0.f;
+#pragma unroll
+  for (int i = 0; i < kSsParts / 2; ++i) {
+    const float4 t = __ldg(p + i);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int k = 2 * i + h;                          // slots merged so far
+      const float mb = h ? t.z : t.x, m2b = h ? t.w : t.y;
+      if (k == 0) { mean = mb; m2 = m2b; continue; }
+      const float d = mb - mean;
+      mean = fmaf(d, 1.f / (float)(k + 1), mean);
+      m2 += fmaf(d * d, 64.f * (float)k / (float)(k + 1), m2b);
+    }
+  }
+  mu = mean;
+  rs = rsqrtf(m2 / (float)g.norm_dim + g.norm_eps);
+}
+
 // ---- epilogues.  Eight epilogue warps: lane quarter q = warp & 3 (the TMEM lanes a warp may read), column half
 // h = (warp - 4) >> 2.  One thread = one accumulator row, half of the tile's columns.  `taddr` carries the quarter.
 template <int BN, int EPI, typename WaitFn>
@@ -94,8 +125,8 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
   const int row = m_blk * BM + row_local;
   const bool valid = row < g.M;
   const bool of16 = g.out_dtype == ZV_F16;
-  if constexpr (EPI != EPI_RESID) wait_accumulator();
-  if constexpr (EPI == EPI_RESID) {
+  if constexpr (!is_resid(EPI) && EPI != EPI_QKV_ROPE_LN && EPI != EPI_QGELU) wait_accumulator();
+  if constexpr (is_resid(EPI)) {
     // X(fp32) += acc + bias, coalesced: the accumulator chunk (32 rows x 32 columns per warp, one row per thread)
     // is transposed through shared memory so that a warp instruction touches 4 rows x 128 contiguous bytes of X
     // (4 L1 wavefronts) instead of 32 rows x 16 bytes (32 wavefronts).  The residual values of a chunk are fetched
@@ -119,6 +150,11 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
     float ssp[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) ssp[i] = 0.f;
+    // EPI_RESID_LN: per row, sums of (x - x0) and (x - x0)^2 over this tile half, x0 = the row's first value in it
+    constexpr bool LN = EPI == EPI_RESID_LN;
+    float x0[8], s1[8], s2[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) x0[i] = s1[i] = s2[i] = 0.f;
     load_x(0);
     wait_accumulator();
 #pragma unroll 1
@@ -144,13 +180,39 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
           *reinterpret_cast<float4*>(xrow + (int64_t)rw * g.ldo + c) = nx;
           if (emit) {
             *reinterpret_cast<uint2*>(x16row + (int64_t)rw * g.N + c) = make_uint2(pack2(nx.x, nx.y, g.op_f16 != 0), pack2(nx.z, nx.w, g.op_f16 != 0));
-            ssp[i] += nx.x * nx.x + nx.y * nx.y + nx.z * nx.z + nx.w * nx.w;
+            if constexpr (!LN) ssp[i] += nx.x * nx.x + nx.y * nx.y + nx.z * nx.z + nx.w * nx.w;
+          }
+        }
+        if constexpr (LN) {
+          if (emit) {                                   // whole warp: rows past M compute values nobody stores
+            const float4 nx = make_float4(xv[i].x + a.x, xv[i].y + a.y, xv[i].z + a.z, xv[i].w + a.w);
+            if (c == 0) x0[i] = __shfl_sync(0xffffffffu, nx.x, lane & ~7);
+            const float dx = nx.x - x0[i], dy = nx.y - x0[i], dz = nx.z - x0[i], dw = nx.w - x0[i];
+            s1[i] += (dx + dy) + (dz + dw);
+            s2[i] += (dx * dx + dy * dy) + (dz * dz + dw * dw);
           }
         }
       }
       if (c + 32 < HALF) load_x(c + 32);
     }
-    if (emit) {
+    if (LN && emit) {
+      // fixed-order butterfly over the row's 8 lanes, then the half's (mean, M2); a 128-column half stores
+      // (mean, M2 / 2) in both of its 64-column slots (merging two equal-mean halves gives back M2 exactly)
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        float a1 = s1[i], a2 = s2[i];
+#pragma unroll
+        for (int o = 1; o < 8; o <<= 1) { a1 += __shfl_xor_sync(0xffffffffu, a1, o); a2 += __shfl_xor_sync(0xffffffffu, a2, o); }
+        const float mean_off = a1 / (float)HALF;
+        const float m2 = fmaxf(fmaf(-a1, mean_off, a2), 0.f);
+        const int rw = 4 * i + rr;
+        if ((lane & 7) == 0 && row_base + rw < g.M) {
+          float2* o = g.ln_out + (int64_t)(row_base + rw) * kSsParts + (n_blk * BN + half * HALF) / 64;
+          if (HALF == 128) { o[0] = o[1] = make_float2(x0[i] + mean_off, 0.5f * m2); }
+          else o[0] = make_float2(x0[i] + mean_off, m2);
+        }
+      }
+    } else if (emit) {
       // the 8 lanes that share a row (lane >> 3) each hold 4 of every 32 columns: fixed-order butterfly, then one
       // lane writes the row's partial for this 128-column half (deterministic: no atomics)
 #pragma unroll
@@ -164,10 +226,15 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
           g.ss_out[(int64_t)(row_base + rw) * kSsParts + (n_blk * BN + half * HALF) / 64] = v;
       }
     }
-  } else if constexpr (EPI == EPI_STORE || EPI == EPI_GELU || EPI == EPI_SCATTER) {
+  } else if constexpr (EPI == EPI_STORE || EPI == EPI_GELU || EPI == EPI_SCATTER || EPI == EPI_QGELU) {
     constexpr int HALF = BN / 2;
     int64_t orow = row;
     bool keep = valid;
+    float mu = 0.f, rs = 1.f;
+    if constexpr (EPI == EPI_QGELU) {
+      row_ln_stats(g, row, valid, mu, rs);              // folded norm2: the row's statistics while the MMAs run
+      wait_accumulator();
+    }
     if constexpr (EPI == EPI_SCATTER) { orow = valid ? (int64_t)__ldg(g.scatter + row) : 0; keep = valid && orow >= 0; }
     const int c_begin = half * HALF;
 #pragma unroll 1
@@ -182,9 +249,17 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = 0.f;
       }
-      tmem_ld_wait();
+      if constexpr (EPI == EPI_QGELU) {
+        float cs[32];
+        load_bias32(g.colsum + n0, cs);
+        tmem_ld_wait();
 #pragma unroll
-      for (int j = 0; j < 32; ++j) v[j] += __uint_as_float(r[j]);
+        for (int j = 0; j < 32; ++j) v[j] = quick_gelu(fmaf(fmaf(-mu, cs[j], __uint_as_float(r[j])), rs, v[j]));
+      } else {
+        tmem_ld_wait();
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] += __uint_as_float(r[j]);
+      }
       if constexpr (EPI == EPI_GELU) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
@@ -261,8 +336,8 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
         for (int j = 0; j < 4; ++j) dst[j] = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
       }
     }
-  } else if constexpr (EPI == EPI_QKV_ROPE) {
-    static_assert(EPI != EPI_QKV_ROPE || BN == 240, "QKV tiles hold three 80-wide heads");
+  } else if constexpr (is_qkv(EPI)) {
+    static_assert(!is_qkv(EPI) || BN == 240, "QKV tiles hold three 80-wide heads");
     // The two warps of a lane quarter split the 40 rotation pairs (d, d+40) of every head 24 : 16 (half 0 owns
     // columns [0,24) + [40,64), half 1 owns [24,40) + [64,80)).  Angle of pair d: pos_h * f_d for d < 20,
     // pos_w * f_(d-20) for d >= 20 (emb = cat(rot, rot), HF :485).  Each thread fetches its row's (cos, sin) pairs ONCE
@@ -283,7 +358,14 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
         ropeS[d * 32 + lane] = pair < 20 ? __ldg(rope_h + pair) : __ldg(rope_w + (pair - 20));
       }
     }
-    const float rs = row_rscale(g, row, valid);
+    float mu = 0.f, rs;
+    if constexpr (EPI == EPI_QKV_ROPE_LN) row_ln_stats(g, row, valid, mu, rs);
+    else rs = row_rscale(g, row, valid);
+    // accumulator of column n with the folded LayerNorm's mean term taken out (EPI_QKV_ROPE: the accumulator itself)
+    auto centred = [&](uint32_t acc, int n) {
+      if constexpr (EPI == EPI_QKV_ROPE_LN) return fmaf(-mu, __ldg(g.colsum + n), __uint_as_float(acc));
+      else return __uint_as_float(acc);
+    };
     wait_accumulator();
     const bool rot_heads_possible = n_blk * 3 < 2 * g.heads;
     const int row0 = m_blk * BM + q * 32;                  // first row of this quarter
@@ -309,9 +391,9 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
         }
         tmem_ld_wait();
 #pragma unroll
-        for (int j = 0; j < 16; ++j) { lo[j] = fmaf(__uint_as_float(l16[j]), rs, lo[j]); hi[j] = fmaf(__uint_as_float(h16[j]), rs, hi[j]); }
+        for (int j = 0; j < 16; ++j) { lo[j] = fmaf(centred(l16[j], n0 + j), rs, lo[j]); hi[j] = fmaf(centred(h16[j], n0 + 40 + j), rs, hi[j]); }
 #pragma unroll
-        for (int j = 0; j < 8; ++j) { lo[16 + j] = fmaf(__uint_as_float(l8[j]), rs, lo[16 + j]); hi[16 + j] = fmaf(__uint_as_float(h8[j]), rs, hi[16 + j]); }
+        for (int j = 0; j < 8; ++j) { lo[16 + j] = fmaf(centred(l8[j], n0 + 16 + j), rs, lo[16 + j]); hi[16 + j] = fmaf(centred(h8[j], n0 + 56 + j), rs, hi[16 + j]); }
       } else {
         uint32_t l16[16], h16[16];
         __syncwarp();
@@ -326,7 +408,7 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int m_blk, int n_b
         }
         tmem_ld_wait();
 #pragma unroll
-        for (int j = 0; j < 16; ++j) { lo[j] = fmaf(__uint_as_float(l16[j]), rs, lo[j]); hi[j] = fmaf(__uint_as_float(h16[j]), rs, hi[j]); }
+        for (int j = 0; j < 16; ++j) { lo[j] = fmaf(centred(l16[j], n0 + 24 + j), rs, lo[j]); hi[j] = fmaf(centred(h16[j], n0 + 64 + j), rs, hi[j]); }
       }
       if (rotate) {
 #pragma unroll
@@ -522,7 +604,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc(const __grid_constant__ C
   } else if (warp >= 4) {
     const int q = warp & 3, half = (warp - 4) >> 2;
     float* xpose = reinterpret_cast<float*>(smem + C::kStages * C::kStageBytes + C::kBarBytes) +
-                   ((EPI == EPI_RESID || EPI == EPI_SCATTER) ? (warp - 4) * (kXposeBytesPerWarp / 4) : 0);   // per-warp area; QKV: the CTA's area
+                   ((is_resid(EPI) || EPI == EPI_SCATTER) ? (warp - 4) * (kXposeBytesPerWarp / 4) : 0);   // per-warp area; QKV: the CTA's area
     int it = 0;
     for (int tile = first_tile; tile < num_tiles; tile += tile_step, ++it) {
       const int m_blk = (tile / n_blocks) * CG + (int)rank, n_blk = tile % n_blocks;
@@ -597,9 +679,10 @@ int launch(const GemmArgs& g, const void* a, int64_t lda, const void* b, int64_t
   cudaError_t e;
   {
     static const char* const kNames[] = {"zv:K2 gemm store", "zv:K2 gemm qkv+rope", "zv:K2 gemm residual", "zv:K2 gemm swiglu",
-                                         "zv:K2 gemm gelu", "zv:K2 gemm scatter"};
+                                         "zv:K2 gemm gelu", "zv:K2 gemm scatter", "zv:K2 gemm qkv+ln+rope",
+                                         "zv:K2 gemm residual+ln", "zv:K2 gemm quickgelu"};
     NvtxRange nvtx(kNames[EPI]);
-    KernelTimer timer(KC_GEMM_STORE + EPI, stream);
+    KernelTimer timer(is_qkv(EPI) ? KC_GEMM_QKV : is_resid(EPI) ? KC_GEMM_RESID : EPI == EPI_QGELU ? KC_GEMM_QGELU : KC_GEMM_STORE + EPI, stream);
     e = launch_pdl(gemm_tc<BN, EPI, CG>, dim3((unsigned)grid), dim3(kThreads), C::kSmemBytes, stream, CG, ta, tb, g);
   }
   count_launch();
@@ -665,6 +748,9 @@ int gemm(int epi, const GemmArgs& g, const void* a, int64_t lda, const void* b, 
       case EPI_SWIGLU: return launch<256, EPI_SWIGLU, 1>(g, a, lda, b, ldb, stream);
       case EPI_GELU: return launch<256, EPI_GELU, 1>(g, a, lda, b, ldb, stream);
       case EPI_SCATTER: return launch<256, EPI_SCATTER, 1>(g, a, lda, b, ldb, stream);
+      case EPI_QKV_ROPE_LN: return launch<240, EPI_QKV_ROPE_LN, 1>(g, a, lda, b, ldb, stream);
+      case EPI_RESID_LN: return launch<256, EPI_RESID_LN, 1>(g, a, lda, b, ldb, stream);
+      case EPI_QGELU: return launch<256, EPI_QGELU, 1>(g, a, lda, b, ldb, stream);
     }
   }
 #endif
@@ -673,17 +759,23 @@ int gemm(int epi, const GemmArgs& g, const void* a, int64_t lda, const void* b, 
       return g.N % 256 == 0 ? launch<256, EPI_STORE, 2>(g, a, lda, b, ldb, stream)
                             : launch<128, EPI_STORE, 1>(g, a, lda, b, ldb, stream);
     case EPI_QKV_ROPE: return launch<240, EPI_QKV_ROPE, 2>(g, a, lda, b, ldb, stream);
-    case EPI_RESID: {
+    case EPI_RESID:
+    case EPI_RESID_LN: {
       // small batches (a single zoom crop: M = 1296): N = 1280 gives 5 column tiles of 256, i.e. 30 CTA pairs of work for
       // 74 pair slots.  128-wide tiles double the parallelism; taken when they cut the wave count x tile width by >= 20 %.
       const int64_t slots = num_sms() / 2, mp = (g.M + 2 * BM - 1) / (2 * BM);
       const int64_t cost256 = 2 * ((mp * (g.N / 256) + slots - 1) / slots), cost128 = (mp * (g.N / 128) + slots - 1) / slots;
-      if (g.N % 256 == 0 && 5 * cost128 > 4 * cost256) return launch<256, EPI_RESID, 2>(g, a, lda, b, ldb, stream);
+      const bool wide = g.N % 256 == 0 && 5 * cost128 > 4 * cost256;
+      if (epi == EPI_RESID_LN)
+        return wide ? launch<256, EPI_RESID_LN, 2>(g, a, lda, b, ldb, stream) : launch<128, EPI_RESID_LN, 2>(g, a, lda, b, ldb, stream);
+      if (wide) return launch<256, EPI_RESID, 2>(g, a, lda, b, ldb, stream);
       return launch<128, EPI_RESID, 2>(g, a, lda, b, ldb, stream);
     }
     case EPI_SWIGLU: return launch<256, EPI_SWIGLU, 2>(g, a, lda, b, ldb, stream);
     case EPI_GELU: return launch<256, EPI_GELU, 2>(g, a, lda, b, ldb, stream);
     case EPI_SCATTER: return launch<256, EPI_SCATTER, 2>(g, a, lda, b, ldb, stream);
+    case EPI_QKV_ROPE_LN: return launch<240, EPI_QKV_ROPE_LN, 2>(g, a, lda, b, ldb, stream);
+    case EPI_QGELU: return launch<256, EPI_QGELU, 2>(g, a, lda, b, ldb, stream);
   }
   return fail(ZV_EINVAL, "gemm: unknown epilogue %d", epi);
 }
@@ -709,6 +801,7 @@ extern "C" int zv_gemm_ex(int32_t epilogue, const void* a_dev, int64_t lda, cons
                           int32_t heads, int32_t op_dtype, void* stream) {
   zv::reset_launch_count();
   if (!a_dev || !b_dev || !out_dev) return zv::fail(ZV_EINVAL, "zv_gemm_ex: null pointer");
+  if (epilogue < zv::EPI_STORE || epilogue > zv::EPI_SCATTER) return zv::fail(ZV_EINVAL, "gemm: unknown epilogue %d", epilogue);
   zv::GemmArgs g{};
   g.M = (int)m; g.N = (int)n; g.K = (int)k;
   g.out = out_dev; g.ldo = ldo; g.out_dtype = out_dtype; g.bias = bias_dev;

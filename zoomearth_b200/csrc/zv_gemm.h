@@ -34,7 +34,12 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
-enum GemmEpilogue { EPI_STORE = 0, EPI_QKV_ROPE = 1, EPI_RESID = 2, EPI_SWIGLU = 3, EPI_GELU = 4, EPI_SCATTER = 5 };
+enum GemmEpilogue { EPI_STORE = 0, EPI_QKV_ROPE = 1, EPI_RESID = 2, EPI_SWIGLU = 3, EPI_GELU = 4, EPI_SCATTER = 5,
+                   // LayerNorm folded into the GEMMs around it (Qwen2-VL tower): separate values so that the
+                   // instantiations above stay exactly as they are
+                   EPI_QKV_ROPE_LN = 6,   // EPI_QKV_ROPE with r * (acc - mu * c_n) + b'_n before the rotary
+                   EPI_RESID_LN = 7,      // EPI_RESID emitting per-slot (mean, M2) instead of sums of squares
+                   EPI_QGELU = 8 };       // quick_gelu(r * (acc - mu * c_n) + b'_n) -> 16-bit (fc1)
 
 struct GemmArgs {
   int M, N, K;
@@ -62,6 +67,14 @@ struct GemmArgs {
   const float* row_ss;
   float norm_eps;
   int norm_dim;
+  // LayerNorm folded the same way (EPI_*_LN, EPI_QGELU), with LN(x) W^T + b = r (x W'^T) - r mu c + b', r = rsqrt(var + eps):
+  //   producer (EPI_RESID_LN): per row and 64-column slot the slot's (mean, M2 = sum of squared deviations) to `ln_out`
+  //     [M][kSsParts] - a 128-column tile half writes its (mean, M2 / 2) into both of its slots, which merge back exactly;
+  //   consumer: `row_ln` [M][kSsParts] merged in slot order (Chan's formula) into the row's mean and variance, and
+  //     `colsum` [N] c_n = sum_k W'[n][k] of the 16-bit weights the MMA multiplies; `bias` is b' = b + W beta.
+  float2* ln_out;
+  const float2* row_ln;
+  const float* colsum;
 };
 constexpr int kSsParts = 20;   // hidden 1280 = 20 x 64 columns (a 256-wide residual tile fills every other one, a 128-wide tile all)
 
@@ -88,6 +101,12 @@ int attention_win_tc(const void* qkv, void* out, int64_t S, int heads, int head_
 int cast_rows_ss(const float* x, void* x16, int x16_f16, float* ss, int64_t rows, int hidden, void* stream);
 // fp32 (S, H) -> bf16 (S, H): y = w * (x * rsqrt(mean(x^2) + eps))   (HF Qwen2_5_VLRMSNorm :66-71)
 int rmsnorm(const float* x, const float* w, void* y, int y_f16, int64_t rows, int hidden, float eps, void* stream);
+// fp32 (S, H) -> 16-bit copy (S, H) + per-row, per-64-column-slot (mean, M2) in ln[row][kSsParts]: the producer side of the
+// folded LayerNorm for the patch-embed output (two-pass per slot)
+int cast_rows_ln(const float* x, void* x16, int x16_f16, float2* ln, int64_t rows, int hidden, void* stream);
+// fp32 (S, H) -> 16-bit (S, H): y = (x - mean) * rsqrt(var + eps) * w + b, two-pass fp32 statistics (torch LayerNorm)
+int layernorm(const float* x, const float* w, const float* b, void* y, int y_f16, int64_t rows, int hidden, float eps,
+              void* stream);
 // patches in HF order (f32 or bf16) -> bf16 in window order (groups of `unit` rows move together)
 int gather_rows(const void* src, int src_dtype, void* dst, int dst_f16, const int32_t* widx, int64_t n_groups, int unit,
                 int cols, void* stream);

@@ -132,7 +132,7 @@ using namespace zv;
 
 extern "C" {
 
-const char* zv_version(void) { return "zoomvit-b200 0.1 (sm_100a)"; }
+const char* zv_version(void) { return "zoomvit-b200 0.2 (sm_100a)"; }
 const char* zv_last_error(void) { return g_err.c_str(); }
 int64_t zv_last_launch_count(void) { return g_launches; }
 

@@ -14,10 +14,22 @@
 //                            H = silu((X16 Wg'^T)/rms+b)*((X16 Wu'^T)/rms+b)       EPI_SWIGLU (gate/up rows interleaved)
 //                            X += H Wd^T + b ; X16, SS                             EPI_RESID
 // Merger (HF :133-146):      Z = rmsnorm(X) viewed (T, 4H); G = gelu(Z W1^T + b); out[widx[i]] = G W2^T + b.
+//
+// Qwen2-VL tower (cfg->tower_kind = ZV_TOWER_QWEN2, HF models/qwen2_vl/modeling_qwen2_vl.py): LayerNorm with gain g and
+// bias beta, folded the same way - LN(x) W^T + b = r (x W'^T) - r mu c + b' with W' = W diag(g) (16-bit), c_n = sum_k W'[n][k]
+// of those rounded weights, b' = b + W beta (fp32, from the fp32 source weights), r = rsqrt(var + eps).  The producers emit
+// per-64-column-slot (mean, M2) (LNS) instead of sums of squares; every block is full attention:
+//                            QKV = rope(r (X16 Wqkv'^T - mu c) + b')   EPI_QKV_ROPE_LN
+//                            A = attention(QKV)                        zv_attn_tc.cu
+//                            X += A Wo^T + b ; X16, LNS                EPI_RESID_LN
+//                            H = quick_gelu(r (X16 W1'^T - mu c) + b') EPI_QGELU   (S, 5120) 16-bit
+//                            X += H W2^T + b ; X16, LNS                EPI_RESID_LN
+// Merger:                    Z = layernorm(X) viewed (T, 4H); then as above.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <map>
@@ -100,6 +112,102 @@ __global__ void __launch_bounds__(256) cast_rows_ss_kernel(const float* __restri
   if (lane < kSsParts) ss[row * kSsParts + lane] = lane == 0 ? s : 0.f;
 }
 
+// One warp per row: 16-bit copy of the row + per 64-column slot its (mean, M2), two-pass (producer side of the folded
+// LayerNorm for the patch-embed output).  Lanes 0-15 hold slot 2j, lanes 16-31 slot 2j+1 of the j-th 128 columns.
+__global__ void __launch_bounds__(256) cast_rows_ln_kernel(const float* __restrict__ x, uint16_t* __restrict__ y, bool f16,
+                                                           float2* __restrict__ ln, int64_t rows, int hidden) {
+  const int64_t row = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (row >= rows) return;
+  ptx::pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const float4* xr = reinterpret_cast<const float4*>(x + row * hidden);
+  uint2* yr = reinterpret_cast<uint2*>(y + row * hidden);
+  for (int j = 0; j < hidden / 128; ++j) {
+    const int idx = 32 * j + lane;
+    const float4 v = xr[idx];
+    yr[idx] = make_uint2(pack2(v.x, v.y, f16), pack2(v.z, v.w, f16));
+    float s = (v.x + v.y) + (v.z + v.w);
+#pragma unroll
+    for (int o = 1; o < 16; o <<= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const float mean = s * (1.f / 64.f);
+    const float dx = v.x - mean, dy = v.y - mean, dz = v.z - mean, dw = v.w - mean;
+    float m2 = (dx * dx + dy * dy) + (dz * dz + dw * dw);
+#pragma unroll
+    for (int o = 1; o < 16; o <<= 1) m2 += __shfl_xor_sync(0xffffffffu, m2, o);
+    if ((lane & 15) == 0) ln[row * kSsParts + 2 * j + (lane >> 4)] = make_float2(mean, m2);
+  }
+}
+
+// One warp per row.  y = (x - mean) * rsqrt(var + eps) * w + b (torch.nn.LayerNorm), two-pass fp32 statistics, 16-bit out.
+__global__ void __launch_bounds__(256) layernorm_kernel(const float* __restrict__ x, const float* __restrict__ w,
+                                                        const float* __restrict__ b, uint16_t* __restrict__ y, bool f16,
+                                                        int64_t rows, int hidden, float eps) {
+  const int64_t row = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (row >= rows) return;
+  ptx::pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const float4* xr = reinterpret_cast<const float4*>(x + row * hidden);
+  const int nv = hidden / 4;
+  float4 v[10];                      // hidden <= 1280
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const int idx = lane + 32 * i;
+    if (idx < nv) { v[i] = xr[idx]; s += (v[i].x + v[i].y) + (v[i].z + v[i].w); }
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  const float mean = s / (float)hidden;
+  float m2 = 0.f;
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const int idx = lane + 32 * i;
+    if (idx < nv) {
+      const float dx = v[i].x - mean, dy = v[i].y - mean, dz = v[i].z - mean, dw = v[i].w - mean;
+      m2 += (dx * dx + dy * dy) + (dz * dz + dw * dw);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) m2 += __shfl_xor_sync(0xffffffffu, m2, o);
+  const float r = rsqrtf(m2 / (float)hidden + eps);
+  const float4* wr = reinterpret_cast<const float4*>(w);
+  const float4* br = reinterpret_cast<const float4*>(b);
+  uint2* yr = reinterpret_cast<uint2*>(y + row * hidden);
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const int idx = lane + 32 * i;
+    if (idx < nv) {
+      const float4 g = __ldg(wr + idx), c = __ldg(br + idx);
+      yr[idx] = make_uint2(pack2(fmaf((v[i].x - mean) * r, g.x, c.x), fmaf((v[i].y - mean) * r, g.y, c.y), f16),
+                           pack2(fmaf((v[i].z - mean) * r, g.z, c.z), fmaf((v[i].w - mean) * r, g.w, c.w), f16));
+    }
+  }
+}
+
+// Folded LayerNorm, weight side.  One warp per output row n of a consumer GEMM: bias[n] += sum_k W[n][k] beta[k] (fp32 from
+// the source weights W) and csum[n] = sum_k W'[n][k] of the packed 16-bit weights (the numbers the MMA multiplies).
+template <typename SrcT, typename PkT>
+__global__ void __launch_bounds__(256) ln_fold_kernel(const SrcT* __restrict__ w, const PkT* __restrict__ wp,
+                                                      const float* __restrict__ beta, float* __restrict__ bias,
+                                                      float* __restrict__ csum, int64_t rows, int64_t cols) {
+  const int64_t n = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (n >= rows) return;
+  const int lane = threadIdx.x & 31;
+  float wb = 0.f, cs = 0.f;
+  for (int64_t k = lane; k < cols; k += 32) {
+    float v;
+    if constexpr (std::is_same<SrcT, float>::value) v = w[n * cols + k];
+    else if constexpr (std::is_same<SrcT, __half>::value) v = __half2float(w[n * cols + k]);
+    else v = __bfloat162float(w[n * cols + k]);
+    wb = fmaf(v, beta[k], wb);
+    if constexpr (std::is_same<PkT, __half>::value) cs += __half2float(wp[n * cols + k]);
+    else cs += __bfloat162float(wp[n * cols + k]);
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) { wb += __shfl_xor_sync(0xffffffffu, wb, o); cs += __shfl_xor_sync(0xffffffffu, cs, o); }
+  if (lane == 0) { bias[n] += wb; csum[n] = cs; }
+}
+
 // dst group i (unit rows x cols, 16-bit operand type) <- src group widx[i] (f32, or already the operand type).
 template <typename SrcT>
 __global__ void __launch_bounds__(256) gather_kernel(const SrcT* __restrict__ src, uint16_t* __restrict__ dst, bool f16,
@@ -156,12 +264,15 @@ __global__ void pack_kernel(const SrcT* __restrict__ src, DstT* __restrict__ dst
 }
 
 // ------------------------------------------------------------------------------------------------ weight layout
-struct LayerOff { int64_t n1, n2, wqkv, bqkv, wo, bo, wgu, bgu, wd, bd; };
+// Qwen2-VL (kind 1): wgu / bgu hold fc1 (inter x H) and its folded bias, wd / bd fc2; n1b / n2b / ln_qb the LayerNorm biases,
+// cqkv / cfc1 the column sums c of the folded weights.
+struct LayerOff { int64_t n1, n2, wqkv, bqkv, wo, bo, wgu, bgu, wd, bd, n1b, n2b, cqkv, cfc1; };
 struct WeightLayout {
   int64_t wpe = 0;
   std::vector<LayerOff> layers;
-  int64_t ln_q = 0, w1 = 0, b1 = 0, w2 = 0, b2 = 0, bytes = 0;
+  int64_t ln_q = 0, w1 = 0, b1 = 0, w2 = 0, b2 = 0, ln_qb = 0, bytes = 0;
 };
+bool qwen2(const zv_cfg* c) { return c->tower_kind == ZV_TOWER_QWEN2; }
 
 WeightLayout weight_layout(const zv_cfg* c) {
   WeightLayout L;
@@ -170,6 +281,20 @@ WeightLayout weight_layout(const zv_cfg* c) {
   auto take = [&](int64_t bytes) { int64_t o = off; off = align_up(off + bytes, 256); return o; };
   L.wpe = take(H * kPatchK * 2);
   L.layers.resize(c->depth);
+  if (qwen2(c)) {
+    for (auto& l : L.layers) {
+      l.n1 = take(H * 4); l.n1b = take(H * 4); l.n2 = take(H * 4); l.n2b = take(H * 4);
+      l.wqkv = take(3 * H * H * 2); l.bqkv = take(3 * H * 4); l.cqkv = take(3 * H * 4);
+      l.wo = take(H * H * 2); l.bo = take(H * 4);
+      l.wgu = take(I * H * 2); l.bgu = take(I * 4); l.cfc1 = take(I * 4);
+      l.wd = take(H * I * 2); l.bd = take(H * 4);
+    }
+    L.ln_q = take(H * 4); L.ln_qb = take(H * 4);
+    L.w1 = take(16 * H * H * 2); L.b1 = take(4 * H * 4);
+    L.w2 = take(O * 4 * H * 2); L.b2 = take(O * 4);
+    L.bytes = off;
+    return L;
+  }
   for (auto& l : L.layers) {
     l.n1 = take(H * 4); l.n2 = take(H * 4);
     l.wqkv = take(3 * H * H * 2); l.bqkv = take(3 * H * 4);
@@ -189,6 +314,16 @@ int check_cfg(const zv_cfg* c, const char* who) {
   if (c->hidden != 1280 || c->heads != 16 || c->out_hidden % 256 || c->patch != 14 || c->merge != 2 || c->temporal != 2 ||
       c->depth < 1 || c->depth > 32 || c->inter <= 0)
     return fail(ZV_EINVAL, "%s: this build covers hidden=1280, heads=16 (head_dim 80), patch=14, merge=2, temporal=2, depth<=32", who);
+  if (c->tower_kind != ZV_TOWER_QWEN25 && c->tower_kind != ZV_TOWER_QWEN2)
+    return fail(ZV_EINVAL, "%s: tower_kind=%d (0 Qwen2.5-VL, 1 Qwen2-VL)", who, c->tower_kind);
+  if (qwen2(c)) {
+    const uint32_t all = c->depth == 32 ? 0xffffffffu : (1u << c->depth) - 1u;
+    if (((uint32_t)c->fullatt_mask_lo & all) != all)
+      return fail(ZV_EINVAL, "%s: tower_kind=1 (Qwen2-VL) has full attention in every block, but fullatt_mask_lo=0x%08x "
+                  "leaves window blocks among the %d", who, (uint32_t)c->fullatt_mask_lo, c->depth);
+    if (c->inter != 5120)
+      return fail(ZV_EINVAL, "%s: tower_kind=1 (Qwen2-VL) needs inter=5120 (fc1 1280 -> 5120), got inter=%d", who, c->inter);
+  }
   return ZV_OK;
 }
 
@@ -223,6 +358,40 @@ int pack_one(const zv_tensor* t, DstT* dst, int64_t rows, int64_t cols, int64_t 
   return ZV_OK;
 }
 
+// Folded LayerNorm bias and column sums of one consumer GEMM (ln_fold_kernel); wp = its packed 16-bit weights.
+int ln_fold(const zv_tensor* t, const void* wp, bool f16, const float* beta, float* bias, float* csum, int64_t rows,
+            int64_t cols, cudaStream_t s) {
+  const unsigned blocks = (unsigned)((rows + 7) / 8);
+#define ZV_FOLD(SRC)                                                                                                     \
+  do {                                                                                                                   \
+    const SRC* w_ = static_cast<const SRC*>(t->data);                                                                   \
+    if (f16) ln_fold_kernel<SRC, __half><<<blocks, 256, 0, s>>>(w_, static_cast<const __half*>(wp), beta, bias, csum, rows, cols); \
+    else ln_fold_kernel<SRC, __nv_bfloat16><<<blocks, 256, 0, s>>>(w_, static_cast<const __nv_bfloat16*>(wp), beta, bias, csum, rows, cols); \
+  } while (0)
+  if (t->dtype == ZV_F32) ZV_FOLD(float);
+  else if (t->dtype == ZV_BF16) ZV_FOLD(__nv_bfloat16);
+  else if (t->dtype == ZV_F16) ZV_FOLD(__half);
+  else return fail(ZV_EINVAL, "zv_weights_pack: %s has unsupported dtype %d", t->name, t->dtype);
+#undef ZV_FOLD
+  count_launch();
+  return ZV_OK;
+}
+
+// Every tensor of the Qwen2-VL tower's state dict (HF names relative to the tower), in packing order.
+std::vector<std::string> qwen2_tensor_names(const zv_cfg* c) {
+  std::vector<std::string> v{"patch_embed.proj.weight"};
+  for (int l = 0; l < c->depth; ++l) {
+    const std::string p = "blocks." + std::to_string(l) + ".";
+    for (const char* n : {"norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias", "attn.qkv.weight", "attn.qkv.bias",
+                          "attn.proj.weight", "attn.proj.bias", "mlp.fc1.weight", "mlp.fc1.bias", "mlp.fc2.weight", "mlp.fc2.bias"})
+      v.push_back(p + n);
+  }
+  for (const char* n : {"merger.ln_q.weight", "merger.ln_q.bias", "merger.mlp.0.weight", "merger.mlp.0.bias",
+                        "merger.mlp.2.weight", "merger.mlp.2.bias"})
+    v.push_back(n);
+  return v;
+}
+
 }  // namespace
 
 int rmsnorm(const float* x, const float* w, void* y, int y_f16, int64_t rows, int hidden, float eps, void* stream) {
@@ -242,6 +411,29 @@ int cast_rows_ss(const float* x, void* x16, int x16_f16, float* ss, int64_t rows
     KernelTimer timer(KC_RMSNORM, stream);
     launch_pdl(cast_rows_ss_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, static_cast<cudaStream_t>(stream), 1,
                x, static_cast<uint16_t*>(x16), x16_f16 != 0, ss, rows, hidden);
+  }
+  count_launch();
+  return ZV_OK;
+}
+
+int cast_rows_ln(const float* x, void* x16, int x16_f16, float2* ln, int64_t rows, int hidden, void* stream) {
+  if (hidden != 64 * kSsParts) return fail(ZV_EINVAL, "cast_rows_ln: hidden=%d unsupported", hidden);
+  {
+    KernelTimer timer(KC_RMSNORM, stream);
+    launch_pdl(cast_rows_ln_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, static_cast<cudaStream_t>(stream), 1,
+               x, static_cast<uint16_t*>(x16), x16_f16 != 0, ln, rows, hidden);
+  }
+  count_launch();
+  return ZV_OK;
+}
+
+int layernorm(const float* x, const float* w, const float* b, void* y, int y_f16, int64_t rows, int hidden, float eps,
+              void* stream) {
+  if (hidden % 4 || hidden > 1280) return fail(ZV_EINVAL, "layernorm: hidden=%d unsupported", hidden);
+  {
+    KernelTimer timer(KC_RMSNORM, stream);
+    launch_pdl(layernorm_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, static_cast<cudaStream_t>(stream), 1,
+               x, w, b, static_cast<uint16_t*>(y), y_f16 != 0, rows, hidden, eps);
   }
   count_launch();
   return ZV_OK;
@@ -291,11 +483,6 @@ int zv_weights_pack(const zv_cfg* cfg, const zv_tensor* tensors, int32_t n, void
   int rc = check_cfg(cfg, "zv_weights_pack");
   if (rc) return rc;
   if (!tensors || !packed_dev) return fail(ZV_EINVAL, "zv_weights_pack: null argument");
-  rc = check_device("zv_weights_pack");
-  if (rc) return rc;
-  const WeightLayout L = weight_layout(cfg);
-  if (packed_bytes < L.bytes) return fail(ZV_ENOMEM, "zv_weights_pack: buffer %lld B < required %lld B", (long long)packed_bytes, (long long)L.bytes);
-  cudaStream_t s = static_cast<cudaStream_t>(stream_);
   std::map<std::string, const zv_tensor*> by_name;
   for (int32_t i = 0; i < n; ++i) {
     std::string nm = tensors[i].name ? tensors[i].name : "";
@@ -303,6 +490,20 @@ int zv_weights_pack(const zv_cfg* cfg, const zv_tensor* tensors, int32_t n, void
       if (nm.rfind(pre, 0) == 0) { nm = nm.substr(std::strlen(pre)); break; }
     by_name[nm] = &tensors[i];
   }
+  if (qwen2(cfg)) {                  // the whole state dict is checked before any device work: missing and extra tensors
+    const std::vector<std::string> names = qwen2_tensor_names(cfg);
+    for (const std::string& nm : names)
+      if (!by_name.count(nm)) return fail(ZV_EINVAL, "zv_weights_pack: missing tensor %s", nm.c_str());
+    for (const auto& kv : by_name)
+      if (std::find(names.begin(), names.end(), kv.first) == names.end())
+        return fail(ZV_EINVAL, "zv_weights_pack: unexpected tensor %s (not part of the Qwen2-VL tower of depth %d)",
+                    kv.first.c_str(), cfg->depth);
+  }
+  rc = check_device("zv_weights_pack");
+  if (rc) return rc;
+  const WeightLayout L = weight_layout(cfg);
+  if (packed_bytes < L.bytes) return fail(ZV_ENOMEM, "zv_weights_pack: buffer %lld B < required %lld B", (long long)packed_bytes, (long long)L.bytes);
+  cudaStream_t s = static_cast<cudaStream_t>(stream_);
   auto get = [&](const std::string& nm) -> const zv_tensor* {
     auto it = by_name.find(nm);
     return it == by_name.end() ? nullptr : it->second;
@@ -312,6 +513,7 @@ int zv_weights_pack(const zv_cfg* cfg, const zv_tensor* tensors, int32_t n, void
   uint8_t* base = static_cast<uint8_t*>(packed_dev);
   const int64_t H = cfg->hidden, I = cfg->inter, IP = ipad(cfg), O = cfg->out_hidden;
   const bool f16 = cfg->op_dtype == ZV_F16;
+#define ZV_TRY_PACK(expr) do { rc = (expr); if (rc) return rc; } while (0)
 #define ZV_PACK_S(NAME, TYPE, OFF, ROWS, COLS, LD, MODE, SCALE)                                            \
   do {                                                                                                      \
     const zv_tensor* t_ = get(NAME);                                                                        \
@@ -324,7 +526,28 @@ int zv_weights_pack(const zv_cfg* cfg, const zv_tensor* tensors, int32_t n, void
   } while (0)
 #define ZV_PACK(NAME, TYPE, OFF, ROWS, COLS, LD, MODE) ZV_PACK_S(NAME, TYPE, OFF, ROWS, COLS, LD, MODE, nullptr)
   ZV_PACK("patch_embed.proj.weight", __nv_bfloat16, L.wpe, H, kPatchK, kPatchK, 0);
-  for (int l = 0; l < cfg->depth; ++l) {
+  auto fl = [&](size_t off) { return reinterpret_cast<float*>(base + off); };
+  for (int l = 0; qwen2(cfg) && l < cfg->depth; ++l) {
+    const std::string p = "blocks." + std::to_string(l) + ".";
+    const LayerOff& o = L.layers[l];
+    ZV_PACK(p + "norm1.weight", float, o.n1, 1, H, H, 0);
+    ZV_PACK(p + "norm1.bias", float, o.n1b, 1, H, H, 0);
+    ZV_PACK(p + "norm2.weight", float, o.n2, 1, H, H, 0);
+    ZV_PACK(p + "norm2.bias", float, o.n2b, 1, H, H, 0);
+    // gains into the weight columns as above; then b' = b + W beta and c = column sums of the packed W'
+    ZV_PACK_S(p + "attn.qkv.weight", __nv_bfloat16, o.wqkv, 3 * H, H, H, 0, fl(o.n1));
+    ZV_PACK(p + "attn.qkv.bias", float, o.bqkv, 1, 3 * H, 3 * H, 0);
+    ZV_TRY_PACK(ln_fold(get(p + "attn.qkv.weight"), base + o.wqkv, f16, fl(o.n1b), fl(o.bqkv), fl(o.cqkv), 3 * H, H, s));
+    ZV_PACK(p + "attn.proj.weight", __nv_bfloat16, o.wo, H, H, H, 0);
+    ZV_PACK(p + "attn.proj.bias", float, o.bo, 1, H, H, 0);
+    ZV_PACK_S(p + "mlp.fc1.weight", __nv_bfloat16, o.wgu, I, H, H, 0, fl(o.n2));
+    ZV_PACK(p + "mlp.fc1.bias", float, o.bgu, 1, I, I, 0);
+    ZV_TRY_PACK(ln_fold(get(p + "mlp.fc1.weight"), base + o.wgu, f16, fl(o.n2b), fl(o.bgu), fl(o.cfc1), I, H, s));
+    ZV_PACK(p + "mlp.fc2.weight", __nv_bfloat16, o.wd, H, I, I, 0);
+    ZV_PACK(p + "mlp.fc2.bias", float, o.bd, 1, H, H, 0);
+  }
+  if (qwen2(cfg)) ZV_PACK("merger.ln_q.bias", float, L.ln_qb, 1, H, H, 0);
+  for (int l = 0; !qwen2(cfg) && l < cfg->depth; ++l) {
     const std::string p = "blocks." + std::to_string(l) + ".";
     const LayerOff& o = L.layers[l];
     ZV_PACK(p + "norm1.weight", float, o.n1, 1, H, H, 0);
@@ -351,13 +574,14 @@ int zv_weights_pack(const zv_cfg* cfg, const zv_tensor* tensors, int32_t n, void
   ZV_PACK("merger.mlp.2.bias", float, L.b2, 1, O, O, 0);
 #undef ZV_PACK
 #undef ZV_PACK_S
+#undef ZV_TRY_PACK
   e = cudaGetLastError();
   if (e != cudaSuccess) return fail(ZV_ECUDA, "zv_weights_pack: %s", cudaGetErrorString(e));
   return ZV_OK;
 }
 
 namespace {
-struct Workspace { int64_t p = 0, x = 0, y = 0, x16 = 0, ss = 0, big = 0, comp = 0, bytes = 0; };
+struct Workspace { int64_t p = 0, x = 0, y = 0, x16 = 0, ss = 0, big = 0, comp = 0, ln = 0, bytes = 0; };
 Workspace workspace_layout(const zv_cfg* c, int64_t S) {
   Workspace w;
   const int64_t H = c->hidden;
@@ -371,6 +595,7 @@ Workspace workspace_layout(const zv_cfg* c, int64_t S) {
   w.ss = take(S * kSsParts * 4);         // per-row partial sums of squares of X (folded RMSNorm)
   w.big = take(S * wide * 2);
   w.comp = take((S / 4 + 1) * 4);        // int32 [T]: composed scatter rows of zv_visual_forward_into
+  if (qwen2(c)) w.ln = take(S * kSsParts * 8);   // float2 [S][kSsParts]: per-slot (mean, M2) of X (folded LayerNorm)
   w.bytes = off;
   return w;
 }
@@ -490,48 +715,86 @@ int visual_forward_impl(const zv_cfg* cfg, const void* weights_dev, const zv_pla
 
   void* X16 = ws + W.x16;
   float* SS = reinterpret_cast<float*>(ws + W.ss);
-  ZV_TRY(cast_rows_ss(X, X16, f16, SS, S, (int)H, stream));
-  for (int l = 0; l < cfg->depth; ++l) {
-    const LayerOff& o = L.layers[l];
-    const bool full = (cfg->fullatt_mask_lo >> l) & 1;
-    g = GemmArgs{};
-    g.op_f16 = f16;
-    g.M = (int)S; g.N = (int)(3 * H); g.K = (int)H; g.out = BIG; g.ldo = 3 * H; g.out_dtype = op;
-    g.bias = reinterpret_cast<const float*>(wb + o.bqkv); g.pos = d_pos; g.rope = d_rope; g.heads = cfg->heads;
-    g.row_ss = SS; g.norm_eps = cfg->eps; g.norm_dim = (int)H;               // norm1 (gain folded into Wqkv)
-    ZV_TRY(gemm(EPI_QKV_ROPE, g, X16, H, wb + o.wqkv, H, stream));
-    if (full && !legacy_full) {
-      ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
-    } else if (!full && !legacy_full) {
-      ZV_TRY(attention_win_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_wblk, p->n_win_blocks, d_wbnd, stream, f16 != 0));
-    } else {
-      ZV_TRY(attention(BIG, Y, cfg->heads, (int)(H / cfg->heads), full ? d_full : d_win, full ? p->n_full_tiles : p->n_win_tiles, stream, full, f16 != 0));
+  if (qwen2(cfg)) {
+    float2* LNS = reinterpret_cast<float2*>(ws + W.ln);
+    ZV_TRY(cast_rows_ln(X, X16, f16, LNS, S, (int)H, stream));
+    for (int l = 0; l < cfg->depth; ++l) {
+      const LayerOff& o = L.layers[l];
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)(3 * H); g.K = (int)H; g.out = BIG; g.ldo = 3 * H; g.out_dtype = op;
+      g.bias = reinterpret_cast<const float*>(wb + o.bqkv); g.pos = d_pos; g.rope = d_rope; g.heads = cfg->heads;
+      g.row_ln = LNS; g.colsum = reinterpret_cast<const float*>(wb + o.cqkv); g.norm_eps = cfg->eps; g.norm_dim = (int)H;   // norm1
+      ZV_TRY(gemm(EPI_QKV_ROPE_LN, g, X16, H, wb + o.wqkv, H, stream));
+      if (!legacy_full) ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
+      else ZV_TRY(attention(BIG, Y, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, true, f16 != 0));
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)H; g.K = (int)H; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
+      g.bias = reinterpret_cast<const float*>(wb + o.bo);
+      g.x16_out = X16; g.ln_out = LNS;
+      ZV_TRY(gemm(EPI_RESID_LN, g, Y, H, wb + o.wo, H, stream));
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)IP; g.K = (int)H; g.out = BIG; g.ldo = IP; g.out_dtype = op;
+      g.bias = reinterpret_cast<const float*>(wb + o.bgu);
+      g.row_ln = LNS; g.colsum = reinterpret_cast<const float*>(wb + o.cfc1); g.norm_eps = cfg->eps; g.norm_dim = (int)H;   // norm2
+      ZV_TRY(gemm(EPI_QGELU, g, X16, H, wb + o.wgu, H, stream));
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)H; g.K = (int)IP; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
+      g.bias = reinterpret_cast<const float*>(wb + o.bd);
+      if (l + 1 < cfg->depth) { g.x16_out = X16; g.ln_out = LNS; }             // the merger normalises in fp32 itself
+      ZV_TRY(gemm(EPI_RESID_LN, g, BIG, IP, wb + o.wd, IP, stream));
     }
-    g = GemmArgs{};
-    g.op_f16 = f16;
-    g.M = (int)S; g.N = (int)H; g.K = (int)H; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
-    g.bias = reinterpret_cast<const float*>(wb + o.bo);
-    g.x16_out = X16; g.ss_out = SS;
-    ZV_TRY(gemm(EPI_RESID, g, Y, H, wb + o.wo, H, stream));
-    g = GemmArgs{};
-    g.op_f16 = f16;
-    g.M = (int)S; g.N = (int)(2 * IP); g.K = (int)H; g.out = BIG; g.ldo = IP; g.out_dtype = op;
-    g.bias = reinterpret_cast<const float*>(wb + o.bgu);
-    g.row_ss = SS; g.norm_eps = cfg->eps; g.norm_dim = (int)H;               // norm2 (gain folded into Wgate / Wup)
-    ZV_TRY(gemm(EPI_SWIGLU, g, X16, H, wb + o.wgu, H, stream));
-    g = GemmArgs{};
-    g.op_f16 = f16;
-    g.M = (int)S; g.N = (int)H; g.K = (int)IP; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
-    g.bias = reinterpret_cast<const float*>(wb + o.bd);
-    if (l + 1 < cfg->depth) { g.x16_out = X16; g.ss_out = SS; }                // the merger normalises in fp32 itself
-    ZV_TRY(gemm(EPI_RESID, g, BIG, IP, wb + o.wd, IP, stream));
+  } else {
+    ZV_TRY(cast_rows_ss(X, X16, f16, SS, S, (int)H, stream));
+    for (int l = 0; l < cfg->depth; ++l) {
+      const LayerOff& o = L.layers[l];
+      const bool full = (cfg->fullatt_mask_lo >> l) & 1;
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)(3 * H); g.K = (int)H; g.out = BIG; g.ldo = 3 * H; g.out_dtype = op;
+      g.bias = reinterpret_cast<const float*>(wb + o.bqkv); g.pos = d_pos; g.rope = d_rope; g.heads = cfg->heads;
+      g.row_ss = SS; g.norm_eps = cfg->eps; g.norm_dim = (int)H;               // norm1 (gain folded into Wqkv)
+      ZV_TRY(gemm(EPI_QKV_ROPE, g, X16, H, wb + o.wqkv, H, stream));
+      if (full && !legacy_full) {
+        ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
+      } else if (!full && !legacy_full) {
+        ZV_TRY(attention_win_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_wblk, p->n_win_blocks, d_wbnd, stream, f16 != 0));
+      } else {
+        ZV_TRY(attention(BIG, Y, cfg->heads, (int)(H / cfg->heads), full ? d_full : d_win, full ? p->n_full_tiles : p->n_win_tiles, stream, full, f16 != 0));
+      }
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)H; g.K = (int)H; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
+      g.bias = reinterpret_cast<const float*>(wb + o.bo);
+      g.x16_out = X16; g.ss_out = SS;
+      ZV_TRY(gemm(EPI_RESID, g, Y, H, wb + o.wo, H, stream));
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)(2 * IP); g.K = (int)H; g.out = BIG; g.ldo = IP; g.out_dtype = op;
+      g.bias = reinterpret_cast<const float*>(wb + o.bgu);
+      g.row_ss = SS; g.norm_eps = cfg->eps; g.norm_dim = (int)H;               // norm2 (gain folded into Wgate / Wup)
+      ZV_TRY(gemm(EPI_SWIGLU, g, X16, H, wb + o.wgu, H, stream));
+      g = GemmArgs{};
+      g.op_f16 = f16;
+      g.M = (int)S; g.N = (int)H; g.K = (int)IP; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
+      g.bias = reinterpret_cast<const float*>(wb + o.bd);
+      if (l + 1 < cfg->depth) { g.x16_out = X16; g.ss_out = SS; }                // the merger normalises in fp32 itself
+      ZV_TRY(gemm(EPI_RESID, g, BIG, IP, wb + o.wd, IP, stream));
+    }
   }
   if (hidden_out_dev) {
     cudaError_t e = cudaMemcpyAsync(hidden_out_dev, X, (size_t)(S * H * 4), cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return fail(ZV_ECUDA, "zv_visual_forward: hidden copy: %s", cudaGetErrorString(e));
   }
-  // merger (HF :133-146) + un-reorder (HF :512-513)
-  ZV_TRY(rmsnorm(X, reinterpret_cast<const float*>(wb + L.ln_q), Y, f16, S, (int)H, cfg->eps, stream));
+  // merger (HF :133-146; Qwen2-VL: LayerNorm ln_q) + un-reorder (HF :512-513)
+  if (qwen2(cfg))
+    ZV_TRY(layernorm(X, reinterpret_cast<const float*>(wb + L.ln_q), reinterpret_cast<const float*>(wb + L.ln_qb), Y, f16, S,
+                     (int)H, cfg->eps, stream));
+  else
+    ZV_TRY(rmsnorm(X, reinterpret_cast<const float*>(wb + L.ln_q), Y, f16, S, (int)H, cfg->eps, stream));
   g = GemmArgs{};
   g.op_f16 = f16;
   g.M = (int)T; g.N = (int)(4 * H); g.K = (int)(4 * H); g.out = BIG; g.ldo = 4 * H; g.out_dtype = op;

@@ -11,12 +11,13 @@ import torch
 import torch.distributed as dist
 
 
-def crop_cost(grid_thw):
-    """FLOP estimate per crop (SURVEY 8e): linear + full attention + window attention."""
+def crop_cost(grid_thw, full_layers=4):
+    """FLOP estimate per crop (SURVEY 8e) of a 32-block tower: linear + full attention + window attention.
+    ``full_layers``: blocks with full attention (4 in Qwen2.5-VL, all 32 in Qwen2-VL); the rest attend in windows."""
     g = np.asarray(grid_thw, dtype=np.float64).reshape(-1, 3)
     S = g[:, 0] * g[:, 1] * g[:, 2]
     T = S / 4
-    return 5.125e9 * T + 4 * 4 * S * S * 1280 + 28 * 4 * 64 * S * 1280
+    return 5.125e9 * T + full_layers * 4 * S * S * 1280 + (32 - full_layers) * 4 * 64 * S * 1280
 
 
 def partition(costs, world_size):
@@ -170,7 +171,9 @@ def encode_sharded(enc, images_dev, boxes, image_index, gather, max_patches=400_
     img_hw = np.array([[images_dev[i].shape[0], images_dev[i].shape[1]] for i in idx], np.int32)
     _, _, grid = geometry.geometry(cfg, img_hw, np.asarray(boxes, np.float64).reshape(n, 4))
     tokens = (grid[:, 0] * grid[:, 1] * grid[:, 2]) // enc.visual.spatial_merge_unit
-    parts = partition(crop_cost(grid), world)
+    from . import _lib
+    full_layers = 32 if enc.visual.cfg.tower_kind == _lib.TOWER_QWEN2 else 4     # Qwen2-VL: every block full attention
+    parts = partition(crop_cost(grid, full_layers), world)
     starts, rows = sharded_rows(parts, tokens)
     if starts[-1] > gather.rows_total:
         raise ValueError(f"gather buffer holds {gather.rows_total} rows, the batch needs {int(starts[-1])}")

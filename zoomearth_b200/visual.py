@@ -20,6 +20,15 @@ _DT = {torch.float32: _lib.ZV_F32, torch.bfloat16: _lib.ZV_BF16, torch.float16: 
 
 
 def _vision_cfg_from_hf(config):
+    """zv_cfg fields of an HF vision config: ``Qwen2_5_VLVisionConfig`` (tower kind 0) or ``Qwen2VLVisionConfig`` (kind 1,
+    whose ``hidden_size`` is the merger's output width and whose blocks are all full attention)."""
+    if getattr(config, "model_type", None) == "qwen2_vl":
+        if config.hidden_act != "quick_gelu":
+            raise NotImplementedError(f"Qwen2-VL tower with hidden_act={config.hidden_act!r}: only quick_gelu is built")
+        return dict(depth=config.depth, hidden=config.embed_dim, heads=config.num_heads,
+                    inter=int(config.embed_dim * config.mlp_ratio), out_hidden=config.hidden_size, patch=config.patch_size,
+                    merge=config.spatial_merge_size, temporal=config.temporal_patch_size,
+                    fullatt=list(range(config.depth)), tower_kind=_lib.TOWER_QWEN2)
     return dict(depth=config.depth, hidden=config.hidden_size, heads=config.num_heads,
                 inter=config.intermediate_size, out_hidden=config.out_hidden_size, patch=config.patch_size,
                 merge=config.spatial_merge_size, temporal=config.temporal_patch_size, window=config.window_size,
@@ -56,6 +65,7 @@ class FusedVisual(nn.Module):
         self._plans = OrderedDict()
         self._graphs = OrderedDict()      # (grid bytes, input dtype, order) -> captured CUDA graph of the tower
         self._ws = None
+        self._rev = {}                    # plan grid bytes -> device reverse index (Qwen2-VL hidden states in HF order)
         self.last_launches = 0
         self._pack(state_dict)
 
@@ -219,6 +229,18 @@ class FusedVisual(nn.Module):
             raise ValueError(f"pixel_values has shape {tuple(x.shape)}, grid_thw implies ({plan.num_patches}, 1176)")
         return x
 
+    def _hf_order(self, hidden, plan):
+        """Window-ordered hidden states (S, hidden) -> HF row order: merge groups of 4 rows gathered by the plan's reverse
+        index.  HF's Qwen2-VL tower never reorders, so its ``last_hidden_state`` is in HF order."""
+        key = plan.grid_thw.tobytes()
+        rev = self._rev.get(key)
+        if rev is None:
+            rev = torch.from_numpy(plan.reverse_index.copy()).to(self._device)
+            self._rev[key] = rev
+            if len(self._rev) > 64:
+                self._rev.pop(next(iter(self._rev)))
+        return hidden.view(-1, self.spatial_merge_unit, hidden.shape[-1]).index_select(0, rev).view(hidden.shape)
+
     def _forward_impl(self, hidden_states, plan, window_order, return_hidden, gather, gather_row, out=None, gather_rows=None):
         """hidden_states: (S, 1176) patches, float32/bfloat16, HF row order (or the window-ordered bf16 output of
         the fused preprocess when ``window_order=True``).  ``gather`` (a ``sharding.PeerGather``) fuses the multi-GPU
@@ -260,6 +282,8 @@ class FusedVisual(nn.Module):
                     _DT[x.dtype], _lib.ORDER_WINDOW if window_order else _lib.ORDER_HF, out.data_ptr(), _DT[self._dtype],
                     hidden.data_ptr() if hidden is not None else None, ws.data_ptr(), ws.numel(), stream))
         self.last_launches = lib.zv_last_launch_count()
+        if hidden is not None and self.cfg.tower_kind == _lib.TOWER_QWEN2:
+            hidden = self._hf_order(hidden, plan)
         if self.return_pooling_output:
             from transformers.modeling_outputs import BaseModelOutputWithPooling
             return BaseModelOutputWithPooling(last_hidden_state=hidden.to(self._dtype), pooler_output=out)
