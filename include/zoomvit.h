@@ -19,10 +19,13 @@
  *   zv_smart_resize       HF:models/qwen2_vl/image_processing_pil_qwen2_vl.py:57-83
  *   zv_geometry           infer.py:41-76 + HF smart_resize + grid computation (pil_qwen2_vl.py:186-187)
  *   zv_resample_*         Pillow ImagingResample coefficient tables (reached from infer.py:84,
- *                         HF:image_transforms.py:368)
- *   zv_normalize_lut      HF:image_transforms.py:89-124 (rescale) + :384-442 (normalize)
+ *                         HF:image_transforms.py:368); by cfg->resample_kind torch's uint8 antialiased bicubic
+ *                         (HF:image_processing_backends.py TorchvisionBackend.resize -> torchvision resize)
+ *   zv_normalize_lut      HF:image_transforms.py:89-124 (rescale) + :384-442 (normalize); by cfg->resample_kind
+ *                         TorchvisionBackend.rescale_and_normalize (rescale folded into mean and std)
  *   zv_preprocess         infer.py:72-75 (Image.crop) + HF:pil_qwen2_vl.py:143-224 (_preprocess: resize,
- *                         rescale, normalize, patchify) as one fused device pass
+ *                         rescale, normalize, patchify) as one fused device pass; by cfg->resample_kind
+ *                         HF:models/qwen2_vl/image_processing_qwen2_vl.py (the torchvision backend) instead
  *   zv_plan_*             HF:models/qwen2_5_vl/modeling_qwen2_5_vl.py:382-409 (rot_pos_emb ids),
  *                         :411-451 (get_window_index), :470-496 (cu_window_seqlens, cu_seqlens)
  *   zv_weights_*          state-dict import of `visual.*` (HF:modeling_qwen2_5_vl.py:345-380 module tree; Qwen2-VL:
@@ -65,6 +68,12 @@ enum { ZV_ORDER_HF = 0, ZV_ORDER_WINDOW = 1 }; /* patch row order: HF merge-grou
  * HF:models/qwen2_vl/modeling_qwen2_vl.py Qwen2VisionTransformerPretrainedModel); requires fullatt_mask_lo to cover all
  * `depth` blocks and inter = 5120. */
 enum { ZV_TOWER_QWEN25 = 0, ZV_TOWER_QWEN2 = 1 };
+/* Resample / normalise convention of zv_preprocess and zv_normalize_lut, i.e. which HF image-processor backend the
+ * pixels match bit for bit.  ZV_RESAMPLE_PIL: Qwen2VLImageProcessorPil (Pillow bicubic, rescale then normalize).
+ * ZV_RESAMPLE_TORCHVISION: Qwen2VLImageProcessor, the transformers 5.x default (torch's uint8 antialiased bicubic:
+ * Pillow's windows and weights quantised to int16 at a per-axis precision; normalize with the rescale folded into
+ * mean and std, in fp32).  zv_resize_u8 is Pillow-only: it stands for the reference's own resize_image. */
+enum { ZV_RESAMPLE_PIL = 0, ZV_RESAMPLE_TORCHVISION = 1 };
 
 /* Processor + model constants (defaults = Qwen2.5-VL-3B vision config + OPENAI_CLIP statistics). */
 typedef struct zv_cfg {
@@ -88,7 +97,7 @@ typedef struct zv_cfg {
   float   eps;          /* 1e-6 */
   float   reserved_f;
   int32_t tower_kind;   /* ZV_TOWER_QWEN25 (zv_default_cfg) or ZV_TOWER_QWEN2 */
-  int32_t reserved_i;
+  int32_t resample_kind; /* ZV_RESAMPLE_PIL (zv_default_cfg) or ZV_RESAMPLE_TORCHVISION */
 } zv_cfg;
 
 ZV_API const char* zv_version(void);
@@ -116,7 +125,12 @@ ZV_API int zv_geometry(const zv_cfg* cfg, int32_t n, const int32_t* img_hw, cons
  * (22-bit fixed point). */
 ZV_API int32_t zv_resample_ksize(int32_t in_size, int32_t out_size);
 ZV_API int zv_resample_coeffs(int32_t in_size, int32_t out_size, int32_t* bounds, int32_t* kk);
-/* lut[3][256] fp32: HF rescale+normalize of every uint8 level. */
+/* Same tables for a resample kind (ZV_RESAMPLE_*), as the kernels consume them: 22-bit taps.  ZV_RESAMPLE_TORCHVISION
+ * taps are torch's int16 taps at the axis precision p, shifted left by 22 - p; *precision = p (22 for Pillow and for a
+ * same-size axis).  Kind ZV_RESAMPLE_PIL equals zv_resample_coeffs. */
+ZV_API int zv_resample_coeffs_ex(int32_t kind, int32_t in_size, int32_t out_size, int32_t* bounds, int32_t* kk,
+                                 int32_t* precision);
+/* lut[3][256] fp32: HF rescale+normalize of every uint8 level, in the arithmetic of cfg->resample_kind. */
 ZV_API int zv_normalize_lut(const zv_cfg* cfg, float* lut768);
 
 /* ---------------------------------------------------------------- device: fused crop->resize->normalize->patchify */
@@ -145,7 +159,8 @@ ZV_API int zv_resize_u8(int32_t n, const uint8_t* const* src_dev, const int32_t*
  * lists of the tensor-core route (csrc/zv_k1_tc.cuh) - over HOST pointers and emulates that route's kernels lane by lane
  * on the CPU.  took_tc[i] = 1 for the crops the route accepts (row pitch a multiple of 4 bytes, <= 4 K blocks per chunk);
  * only those are written.  u8_dst_host == NULL: fp32 patches into out_host (zv_preprocess), else uint8 images
- * (zv_resize_u8).  Checks everything but the hardware layouts (swizzle, descriptors, TMEM), which the GPU tests cover. */
+ * (zv_resize_u8).  The tables follow cfg->resample_kind (cfg may be NULL in uint8 mode: Pillow's).  Checks everything but
+ * the hardware layouts (swizzle, descriptors, TMEM), which the GPU tests cover. */
 ZV_API int zv_debug_k1_tc_host(const zv_cfg* cfg, int32_t n, const uint8_t* const* src_host, const int32_t* src_hw,
                                const int64_t* src_pitch, const int32_t* crop_box, const int32_t* resized_hw, float* out_host,
                                int32_t row_order, uint8_t* const* u8_dst_host, const int64_t* u8_pitch, void* workspace_host,

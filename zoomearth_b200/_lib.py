@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libzoomvit.so")
 ZV_F32, ZV_BF16, ZV_F16 = 0, 1, 2
 ORDER_HF, ORDER_WINDOW = 0, 1
 TOWER_QWEN25, TOWER_QWEN2 = 0, 1
+RESAMPLE_PIL, RESAMPLE_TORCHVISION = 0, 1
 ZV_EINVAL, ZV_EINVAL_ASPECT, ZV_EINVAL_BOX, ZV_ENOMEM, ZV_ECUDA, ZV_ENODEV, ZV_EARCH = -1, -2, -3, -4, -5, -6, -7
 
 
@@ -22,7 +23,7 @@ class ZvCfg(C.Structure):
         ("inter", C.c_int32), ("out_hidden", C.c_int32), ("fullatt_mask_lo", C.c_int32), ("op_dtype", C.c_int32),
         ("min_pixels", C.c_int64), ("max_pixels", C.c_int64), ("rescale", C.c_double),
         ("mean", C.c_float * 3), ("std", C.c_float * 3), ("eps", C.c_float), ("reserved_f", C.c_float),
-        ("tower_kind", C.c_int32), ("reserved_i", C.c_int32),
+        ("tower_kind", C.c_int32), ("resample_kind", C.c_int32),
     ]
 
 
@@ -54,6 +55,7 @@ _PROTOS = {
     "zv_geometry": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zv_resample_ksize": (C.c_int32, [C.c_int32, C.c_int32]),
     "zv_resample_coeffs": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "zv_resample_coeffs_ex": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, _P(C.c_int32)]),
     "zv_normalize_lut": (C.c_int, [_P(ZvCfg), C.c_void_p]),
     "zv_preprocess_workspace_bytes": (C.c_int64, [C.c_int32, C.c_void_p, C.c_void_p]),
     "zv_preprocess": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -50,11 +50,13 @@ class KernelTimer {
 struct AxisCoeffs {
   int32_t in_size = 0, out_size = 0, ksize = 0;
   std::vector<int32_t> bounds;   // [out][2]
-  std::vector<int32_t> kk;       // [out][ksize]
+  std::vector<int32_t> kk;       // [out][ksize], 22-bit fixed point
+  int32_t precision = 22;        // bits of the taps before they were moved to 22 bits (ZV_RESAMPLE_TORCHVISION: p)
 };
 int32_t resample_ksize(int32_t in_size, int32_t out_size);
-void resample_coeffs(int32_t in_size, int32_t out_size, AxisCoeffs* out);
-void normalize_lut(const zv_cfg* cfg, float* lut768);
+int check_resample_kind(int32_t kind, const char* who);   // ZV_OK, or ZV_EINVAL with a message
+void resample_coeffs(int32_t kind, int32_t in_size, int32_t out_size, AxisCoeffs* out);
+void normalize_lut(const zv_cfg* cfg, float* lut768);      // in the arithmetic of cfg->resample_kind
 void plan_device_image(const zv_plan* p, std::vector<uint8_t>* image);
 void build_window_blocks(const std::vector<int32_t>& cu, int32_t max_rows, std::vector<int32_t>* blocks);
 void fill_window_bounds(const std::vector<int32_t>& cu, int32_t* bounds);

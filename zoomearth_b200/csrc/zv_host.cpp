@@ -5,7 +5,8 @@
 //   cut_box        reference src/eval/infer.py:41-76
 //   resize_dims    reference src/eval/infer.py:78-85
 //   smart_resize   HF models/qwen2_vl/image_processing_pil_qwen2_vl.py:57-83
-//   coefficients   Pillow ImagingResample (precompute_coeffs + normalize_coeffs_8bpc), bicubic a=-0.5
+//   coefficients   Pillow ImagingResample (precompute_coeffs + normalize_coeffs_8bpc), bicubic a=-0.5; or torch's
+//                  uint8 antialiased bicubic (aten UpSampleKernel.cpp, int16 taps), what torchvision's resize runs
 //   plan           HF models/qwen2_5_vl/modeling_qwen2_5_vl.py:382-451,470-496
 #include <algorithm>
 #include <cmath>
@@ -54,20 +55,12 @@ int32_t resample_ksize(int32_t in_size, int32_t out_size) {
   return (int32_t)std::ceil(2.0 * fs) * 2 + 1;
 }
 
-void resample_coeffs(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
-  c->in_size = in_size;
-  c->out_size = out_size;
-  c->ksize = resample_ksize(in_size, out_size);
-  c->bounds.assign((size_t)out_size * 2, 0);
-  c->kk.assign((size_t)out_size * c->ksize, 0);
-  if (in_size == out_size) {                       // same size: Pillow copies, expressed as one exact tap
-    for (int32_t xx = 0; xx < out_size; ++xx) {
-      c->bounds[2 * xx] = xx;
-      c->bounds[2 * xx + 1] = 1;
-      c->kk[xx] = 1 << 22;
-    }
-    return;
-  }
+int check_resample_kind(int32_t kind, const char* who) {
+  if (kind == ZV_RESAMPLE_PIL || kind == ZV_RESAMPLE_TORCHVISION) return ZV_OK;
+  return fail(ZV_EINVAL, "%s: resample_kind %d (0 ZV_RESAMPLE_PIL, 1 ZV_RESAMPLE_TORCHVISION)", who, kind);
+}
+
+static void resample_coeffs_pil(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
   const double scale = (double)in_size / out_size;
   const double fs = scale < 1.0 ? 1.0 : scale;
   const double support = 2.0 * fs;
@@ -97,6 +90,62 @@ void resample_coeffs(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
   }
 }
 
+// torch's taps: Pillow's windows (clamped to ksize) and fp64 weights, rounded to int16 at ONE precision p for the whole
+// axis - the first p < 22 at which the largest weight would need 16 bits one bit further - then moved to 22 bits.  A tap
+// t 2^(22-p) makes the kernels' (acc + 2^21) >> 22 equal to torch's (acc_p + 2^(p-1)) >> p, so every K1 route runs them.
+static void resample_coeffs_tv(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
+  const double scale = (double)in_size / out_size;
+  const double support = scale >= 1.0 ? 2.0 * scale : 2.0;
+  const double invscale = scale >= 1.0 ? 1.0 / scale : 1.0;
+  const int32_t ks = c->ksize;
+  std::vector<double> w((size_t)out_size * ks, 0.0);
+  double w_max = 0.0;
+  for (int32_t xx = 0; xx < out_size; ++xx) {
+    const double center = scale * (xx + 0.5);
+    const int32_t xmin = std::max((int32_t)(center - support + 0.5), 0);
+    const int32_t xsize = std::min(std::max(std::min((int32_t)(center + support + 0.5), in_size) - xmin, 0), ks);
+    double* wx = &w[(size_t)xx * ks];
+    double total = 0.0;
+    for (int32_t j = 0; j < xsize; ++j) {
+      wx[j] = bicubic((j + xmin - center + 0.5) * invscale);
+      total += wx[j];
+    }
+    if (total != 0.0)
+      for (int32_t j = 0; j < xsize; ++j) {
+        wx[j] /= total;
+        w_max = std::max(w_max, wx[j]);
+      }
+    c->bounds[2 * xx] = xmin;
+    c->bounds[2 * xx + 1] = xsize;
+  }
+  int32_t p = 0;
+  while (p < 22 && (int32_t)(0.5 + w_max * (double)(1 << (p + 1))) < (1 << 15)) ++p;
+  c->precision = p;
+  for (size_t i = 0; i < w.size(); ++i) {
+    const double v = w[i] * (double)(1 << p);
+    c->kk[i] = (v < 0 ? (int32_t)(-0.5 + v) : (int32_t)(0.5 + v)) * (1 << (22 - p));
+  }
+}
+
+void resample_coeffs(int32_t kind, int32_t in_size, int32_t out_size, AxisCoeffs* c) {
+  c->in_size = in_size;
+  c->out_size = out_size;
+  c->ksize = resample_ksize(in_size, out_size);
+  c->bounds.assign((size_t)out_size * 2, 0);
+  c->kk.assign((size_t)out_size * c->ksize, 0);
+  c->precision = 22;
+  if (in_size == out_size) {                       // same size: both libraries skip the pass, expressed as one exact tap
+    for (int32_t xx = 0; xx < out_size; ++xx) {
+      c->bounds[2 * xx] = xx;
+      c->bounds[2 * xx + 1] = 1;
+      c->kk[xx] = 1 << 22;
+    }
+    return;
+  }
+  if (kind == ZV_RESAMPLE_TORCHVISION) resample_coeffs_tv(in_size, out_size, c);
+  else resample_coeffs_pil(in_size, out_size, c);
+}
+
 // Row blocks of the tcgen05 window-attention kernel: windows (segments of cu, each <= max_rows) in order, as many whole
 // consecutive ones per block as fit in max_rows rows.  4 ints per block: (row0, n_rows, 0, 0).
 void build_window_blocks(const std::vector<int32_t>& cu, int32_t max_rows, std::vector<int32_t>* blocks) {
@@ -119,6 +168,15 @@ void fill_window_bounds(const std::vector<int32_t>& cu, int32_t* bounds) {
 }
 
 void normalize_lut(const zv_cfg* cfg, float* lut) {
+  if (cfg->resample_kind == ZV_RESAMPLE_TORCHVISION) {
+    // TorchvisionBackend.rescale_and_normalize: mean' = f32(mean) * f32(1 / rescale), std' likewise, (f32(v) - mean') / std'
+    const float inv = (float)(1.0 / cfg->rescale);
+    for (int c = 0; c < 3; ++c) {
+      const float m = cfg->mean[c] * inv, s = cfg->std[c] * inv;
+      for (int v = 0; v < 256; ++v) lut[c * 256 + v] = ((float)v - m) / s;
+    }
+    return;
+  }
   for (int c = 0; c < 3; ++c)
     for (int v = 0; v < 256; ++v) {
       float x = (float)((double)v * cfg->rescale);      // rescale: f64 product, then cast to f32
@@ -132,7 +190,7 @@ using namespace zv;
 
 extern "C" {
 
-const char* zv_version(void) { return "zoomvit-b200 0.2 (sm_100a)"; }
+const char* zv_version(void) { return "zoomvit-b200 0.3 (sm_100a)"; }
 const char* zv_last_error(void) { return g_err.c_str(); }
 int64_t zv_last_launch_count(void) { return g_launches; }
 
@@ -282,15 +340,25 @@ int32_t zv_resample_ksize(int32_t in_size, int32_t out_size) {
 
 int zv_resample_coeffs(int32_t in_size, int32_t out_size, int32_t* bounds, int32_t* kk) {
   if (in_size <= 0 || out_size <= 0 || !bounds || !kk) return fail(ZV_EINVAL, "zv_resample_coeffs: bad argument");
+  return zv_resample_coeffs_ex(ZV_RESAMPLE_PIL, in_size, out_size, bounds, kk, nullptr);
+}
+
+int zv_resample_coeffs_ex(int32_t kind, int32_t in_size, int32_t out_size, int32_t* bounds, int32_t* kk, int32_t* precision) {
+  if (in_size <= 0 || out_size <= 0 || !bounds || !kk) return fail(ZV_EINVAL, "zv_resample_coeffs_ex: bad argument");
+  int rc = check_resample_kind(kind, "zv_resample_coeffs_ex");
+  if (rc) return rc;
   AxisCoeffs c;
-  resample_coeffs(in_size, out_size, &c);
+  resample_coeffs(kind, in_size, out_size, &c);
   std::memcpy(bounds, c.bounds.data(), c.bounds.size() * sizeof(int32_t));
   std::memcpy(kk, c.kk.data(), c.kk.size() * sizeof(int32_t));
+  if (precision) *precision = c.precision;
   return ZV_OK;
 }
 
 int zv_normalize_lut(const zv_cfg* cfg, float* lut) {
   if (!cfg || !lut) return fail(ZV_EINVAL, "zv_normalize_lut: null argument");
+  int rc = check_resample_kind(cfg->resample_kind, "zv_normalize_lut");
+  if (rc) return rc;
   normalize_lut(cfg, lut);
   return ZV_OK;
 }

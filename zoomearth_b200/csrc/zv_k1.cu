@@ -40,6 +40,7 @@
 #include <map>
 #include <memory>
 #include <mutex>
+#include <tuple>
 #include <type_traits>
 #include <vector>
 
@@ -764,11 +765,13 @@ inline int32_t tc_k_blocks(const zv::AxisCoeffs& ac, int32_t n_out, int32_t ch) 
 // B variants of an input with this row pitch: distinct values of (q pitch) mod 16 over the four row phases
 inline int32_t tc_variants(int64_t pitch) { return (pitch & 15) == 0 ? 1 : (pitch & 7) == 0 ? 2 : 4; }
 std::mutex g_axis_mu;
-std::map<std::pair<int32_t, int32_t>, std::shared_ptr<const AxisCache>> g_axis_cache;
+std::map<std::tuple<int32_t, int32_t, int32_t>, std::shared_ptr<const AxisCache>> g_axis_cache;   // (resample kind, in, out)
 
 // Workspace layout shared by zv_preprocess_workspace_bytes and zv_preprocess.
 // u8_out: the vertical pass writes plain uint8 images (zv_resize_u8): any positive output size, row-group work items.
-int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, Layout* L, bool fill, bool u8_out = false) {
+// kind (ZV_RESAMPLE_*) selects the taps; the layout itself depends on the geometry alone.
+int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, Layout* L, bool fill, bool u8_out = false,
+                 int32_t kind = ZV_RESAMPLE_PIL) {
   L->tmp_off.resize(n); L->ybox0.resize(n); L->nrows.resize(n); L->u_off.resize(n); L->t_pitch.resize(n);
   int64_t coef_ints = 0, tmp_bytes = 0;
   for (int32_t i = 0; i < n; ++i) {
@@ -791,12 +794,13 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
       t.off_mma = (int32_t)(coef_ints + 2 * (int64_t)key.second + (int64_t)key.second * t.ksize + (int64_t)key.second * (1 + 3 * t.nw));
       const int64_t ints = 2 * (int64_t)key.second + (int64_t)key.second * t.ksize + (int64_t)key.second * (1 + 3 * t.nw) +
                            (t.ks_mma ? n_blk8 * (1 + 192 * t.ks_mma) : 0);
-      // the tables of an axis depend on (in, out) alone: built once per process and geometry, then copied - a zoom loop
-      // asks for the same few sizes over and over and the fp64 tap generation would otherwise pace every small call
+      // the tables of an axis depend on (kind, in, out) alone: built once per process and geometry, then copied - a zoom
+      // loop asks for the same few sizes over and over and the fp64 tap generation would otherwise pace every small call
+      const std::tuple<int32_t, int32_t, int32_t> ckey{kind, key.first, key.second};
       std::shared_ptr<const AxisCache> hit;
       if (fill) {
         std::lock_guard<std::mutex> lock(g_axis_mu);
-        auto itc = g_axis_cache.find(key);
+        auto itc = g_axis_cache.find(ckey);
         if (itc != g_axis_cache.end()) hit = itc->second;
       }
       if (fill && hit) {
@@ -806,7 +810,7 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
       } else if (fill) {
         const size_t coef_start = L->coef.size();
         zv::AxisCoeffs ac;
-        zv::resample_coeffs(key.first, key.second, &ac);
+        zv::resample_coeffs(kind, key.first, key.second, &ac);
         L->coef.insert(L->coef.end(), ac.bounds.begin(), ac.bounds.end());
         L->coef.insert(L->coef.end(), ac.kk.begin(), ac.kk.end());
         // dp4a limb table: the window starts at the first tap rounded down to 4 samples
@@ -890,7 +894,7 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
         entry->nkb3 = t.nkb3; entry->nkb1 = t.nkb1;
         std::lock_guard<std::mutex> lock(g_axis_mu);
         if (g_axis_cache.size() >= 512) g_axis_cache.clear();              // bounded: a few hundred KB per entry at most
-        g_axis_cache[key] = entry;
+        g_axis_cache[ckey] = entry;
       }
       L->axis[key] = t;
       coef_ints += ints;
@@ -1034,11 +1038,15 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
   // tensor-core route's kernels are emulated on the CPU over the very tables built here and emulate_tc[i] tells which
   // crops took that route (the others are left untouched).
   const bool u8_out = u8_dst != nullptr;
+  // zv_resize_u8 passes no cfg: it is the reference's Pillow resize_image
+  const int32_t kind = cfg ? cfg->resample_kind : ZV_RESAMPLE_PIL;
+  int rc = zv::check_resample_kind(kind, who);
+  if (rc) return rc;
   int ndev = 0;
   if (!emulate_tc && (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)) return zv::fail(ZV_ENODEV, "%s: no CUDA device", who);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   Layout L;
-  int rc = build_layout(n, crop_box, resized_hw, &L, true, u8_out);
+  rc = build_layout(n, crop_box, resized_hw, &L, true, u8_out, kind);
   if (rc) return rc;
   if (workspace_bytes < L.bytes)
     return zv::fail(ZV_ENOMEM, "%s: workspace %lld B < required %lld B", who, (long long)workspace_bytes, (long long)L.bytes);

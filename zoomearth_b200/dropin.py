@@ -4,6 +4,10 @@ After this, the reference's own scripts run unchanged on top of the drop-in: ``p
 (``src/eval/infer.py:102-107``, ``src/demo.py:7-12``) lands on FusedImageProcessor, and the LM forward's
 ``self.visual(pixel_values, grid_thw=...)`` (HF modeling_qwen2_5_vl.py:1172) lands on FusedVisual.  The module
 path is ``model.visual`` on transformers 4.49 (what the reference pins) and ``model.model.visual`` on 5.x.
+
+``image_backend`` picks the HF image-processor backend whose pixels the fused processor reproduces.  On transformers
+5.x ``AutoProcessor`` hands Qwen2-VL / Qwen2.5-VL the torchvision backend whenever torchvision is installed, so a 5.x
+user who wants the model to keep seeing the same ``pixel_values`` passes ``image_backend="match"``.
 """
 import torch
 
@@ -18,9 +22,50 @@ def _find_visual(model):
     raise AttributeError("no `.visual` / `.model.visual` on this model")
 
 
-def install(model=None, processor=None, device=None, dtype=None):
-    """Returns (fused_visual or None, fused_image_processor or None)."""
+def _bicubic(resample):
+    try:
+        from torchvision.transforms import InterpolationMode
+        if resample == InterpolationMode.BICUBIC:
+            return True
+    except ImportError:                     # pragma: no cover
+        pass
+    return isinstance(resample, int) and int(resample) == 3      # PILImageResampling.BICUBIC
+
+
+def _image_backend(old, image_backend):
+    """The FusedImageProcessor backend for ``install(..., image_backend=...)`` replacing the image processor ``old``."""
+    if image_backend not in ("pil", "torchvision", "match"):
+        raise ValueError(f"image_backend must be 'pil', 'torchvision' or 'match', got {image_backend!r}")
+    if image_backend == "pil":
+        return "pil"
+    backend = image_backend
+    if image_backend == "match":
+        try:
+            from transformers.image_processing_backends import PilBackend, TorchvisionBackend
+        except ImportError:
+            PilBackend = TorchvisionBackend = ()
+        if TorchvisionBackend and isinstance(old, TorchvisionBackend):
+            backend = "torchvision"
+        elif PilBackend and isinstance(old, PilBackend):
+            backend = "pil"
+        else:
+            raise ValueError(f"image_backend='match': cannot tell which backend {type(old).__name__} resamples with "
+                             "(known: transformers 5.x TorchvisionBackend / PilBackend); pass 'pil' or 'torchvision'")
+    resample = getattr(old, "resample", None)
+    if not _bicubic(resample):
+        raise NotImplementedError(f"{type(old).__name__} resamples with {resample!r}; the fused processor reproduces "
+                                  "bicubic only")
+    return backend
+
+
+def install(model=None, processor=None, device=None, dtype=None, image_backend="pil"):
+    """Returns (fused_visual or None, fused_image_processor or None).  ``image_backend``: "pil" (the default) matches
+    HF's PIL backend; "torchvision" matches HF's torchvision backend; "match" reads which of the two
+    ``processor.image_processor`` is (a transformers 5.x ``TorchvisionBackend`` or ``PilBackend`` instance, anything else
+    is a ValueError).  Under "torchvision" / "match" a replaced processor that does not resample bicubic raises
+    NotImplementedError."""
     fv = fp = None
+    backend = _image_backend(processor.image_processor, image_backend) if processor is not None else None
     if model is not None:
         owner = _find_visual(model)
         hf_visual = owner.visual
@@ -38,6 +83,6 @@ def install(model=None, processor=None, device=None, dtype=None):
                                  temporal_patch_size=getattr(old, "temporal_patch_size", 2),
                                  merge_size=getattr(old, "merge_size", 2),
                                  image_mean=getattr(old, "image_mean", None), image_std=getattr(old, "image_std", None),
-                                 device=device)
+                                 device=device, backend=backend)
         processor.image_processor = fp
     return fv, fp

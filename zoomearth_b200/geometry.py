@@ -124,6 +124,18 @@ def resample_coeffs(in_size, out_size):
     return ks, bounds, kk
 
 
+def resample_coeffs_ex(kind, in_size, out_size):
+    """The 22-bit taps K1 runs for resample kind ``kind`` (``_lib.RESAMPLE_*``): (ksize, bounds, kk, precision), where
+    precision is the axis precision of torchvision's int16 taps (22 for Pillow and same-size axes)."""
+    ks = _lib.check(_lib.lib().zv_resample_ksize(int(in_size), int(out_size)))
+    bounds = np.empty((out_size, 2), np.int32)
+    kk = np.empty((out_size, ks), np.int32)
+    p = C.c_int32(0)
+    _lib.check(_lib.lib().zv_resample_coeffs_ex(int(kind), int(in_size), int(out_size), bounds.ctypes.data, kk.ctypes.data,
+                                                C.byref(p)))
+    return ks, bounds, kk, p.value
+
+
 def normalize_lut(cfg):
     lut = np.empty((3, 256), np.float32)
     _lib.check(_lib.lib().zv_normalize_lut(C.byref(cfg), lut.ctypes.data))

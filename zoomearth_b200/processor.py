@@ -5,7 +5,11 @@ Replaces ``processor.image_processor`` of ``Qwen2_5_VLProcessor`` (reference cal
 (``pixel_values (S,1176) float32``, ``image_grid_thw (N,3) int64``), same attributes the processor reads
 (``merge_size`` HF processing_qwen2_5_vl.py:120, ``get_number_of_image_patches`` :168, ``model_input_names``).
 What it replaces inside: HF ``models/qwen2_vl/image_processing_pil_qwen2_vl.py:143-224`` (smart_resize ->
-Pillow bicubic -> rescale -> normalize -> patchify); results are bit-identical to that PIL backend.
+Pillow bicubic -> rescale -> normalize -> patchify); results are bit-identical to that PIL backend.  With
+``backend="torchvision"`` they are bit-identical to HF's torchvision backend instead
+(``models/qwen2_vl/image_processing_qwen2_vl.py``, what ``AutoImageProcessor`` returns on transformers 5.x when
+torchvision is installed): torch's uint8 antialiased bicubic and the fp32 fused rescale + normalize.  The device
+kernels are the same; only the coefficient tables and the normalisation LUT differ.
 
 Also the crop-aware entry ``preprocess_crops`` used by the zoom fast path: the source image stays resident on
 the GPU as uint8 and every zoom step reads its crop box straight out of it (``Image.crop`` semantics of
@@ -98,13 +102,22 @@ def _to_u8_hwc(image):
     return image.contiguous()
 
 
+BACKENDS = {"pil": _lib.RESAMPLE_PIL, "torchvision": _lib.RESAMPLE_TORCHVISION}
+
+
 class FusedImageProcessor:
     model_input_names = ["pixel_values", "image_grid_thw"]
     valid_kwargs = None
 
     def __init__(self, min_pixels=None, max_pixels=None, size=None, patch_size=14, temporal_patch_size=2,
                  merge_size=2, image_mean=None, image_std=None, rescale_factor=1 / 255, device=None,
-                 output_device="cpu", **unused):
+                 output_device="cpu", backend="pil", **unused):
+        """``backend``: which HF image-processor backend the pixels match bit for bit - "pil" (Qwen2VLImageProcessorPil)
+        or "torchvision" (Qwen2VLImageProcessor).  It applies to ``preprocess`` / ``__call__`` and ``preprocess_crops``;
+        ``resize_u8`` / ``cut_resize`` are the reference's own Pillow ``resize_image`` under either."""
+        if backend not in BACKENDS:
+            raise ValueError(f"backend must be one of {sorted(BACKENDS)}, got {backend!r}")
+        self.backend = backend
         size = dict(size) if size is not None else {"shortest_edge": 56 * 56, "longest_edge": 28 * 28 * 1280}
         if min_pixels is not None:
             size["shortest_edge"] = min_pixels
@@ -144,7 +157,8 @@ class FusedImageProcessor:
         return _lib.default_cfg(patch=self.patch_size, merge=self.merge_size, temporal=self.temporal_patch_size,
                                 min_pixels=int(min_pixels if min_pixels is not None else self.min_pixels),
                                 max_pixels=int(max_pixels if max_pixels is not None else self.max_pixels),
-                                rescale=float(self.rescale_factor), mean=self.image_mean, std=self.image_std)
+                                rescale=float(self.rescale_factor), mean=self.image_mean, std=self.image_std,
+                                resample_kind=BACKENDS[self.backend])
 
     def _device(self):
         if self.device is None:
