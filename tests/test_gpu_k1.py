@@ -31,6 +31,7 @@ CASES = [
     (640, 28, None, 3136, 12845056, "thin image"),
     (1203, 1600, None, 3136, 1003520, "height not a multiple of 4: the last rows come through the end-aligned tensor map"),
     (1203, 1600, (40, 700, 1500, 1203), 3136, 12845056, "crop that ends on the image's last row, height = 3 mod 4"),
+    (1220, 1220, None, 3136, 50176, "row pitch 12 mod 16 at 5.45x: the tensor-core route declines, the dp4a pass takes what IMMA took"),
 ]
 
 

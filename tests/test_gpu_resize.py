@@ -28,21 +28,25 @@ def proc(cuda):
 
 
 def test_resize_u8_bitexact_vs_live_pillow(cuda, proc):
-    """Crop boxes inside / outside the image, down- and up-scales, same-size axes (Pillow copies), odd widths, every tap
-    class of the dp4a path (5 .. 45 taps) and the per-tap path (> 45 taps)."""
+    """Crop boxes inside / outside the image, down- and up-scales, same-size axes (Pillow copies), odd widths, 5 .. > 45
+    taps on the per-tap path (the 1803-pixel rows, 5409 bytes, are not 4-byte aligned), and the dp4a path on a second image
+    whose 1220-pixel rows are (3660 bytes, 12 mod 16: the tensor-core route declines its 5.45x downscale)."""
     from PIL import Image
     rng = np.random.default_rng(21)
     img = rng.integers(0, 256, (1237, 1803, 3), dtype=np.uint8)
-    dev = torch.from_numpy(img).to(cuda)
-    pil = Image.fromarray(img)
+    img2 = rng.integers(0, 256, (1220, 1220, 3), dtype=np.uint8)
+    devs = [torch.from_numpy(img).to(cuda), torch.from_numpy(img2).to(cuda)]
+    pils = [Image.fromarray(img), Image.fromarray(img2)]
     cases = [((0, 0, 1803, 1237), (512, 351)), ((10, 20, 1310, 920), (512, 354)), ((100, 100, 612, 612), (504, 504)),
              ((0, 0, 600, 600), (600, 300)), ((0, 0, 600, 600), (300, 600)), ((-30, -20, 200, 150), (140, 112)),
              ((5, 5, 33, 33), (56, 56)), ((1700, 1100, 1900, 1300), (333, 77)), ((0, 0, 1803, 1237), (1803, 1237)),
              ((3, 7, 1000, 1200), (997, 1193)), ((0, 0, 1803, 1237), (41, 29)), ((0, 0, 1803, 1237), (17, 1237)),
              ((200, 300, 1229, 811), (1024, 509)), ((0, 0, 1800, 1236), (2048, 1406))]
-    outs = proc.resize_u8([dev], [b for b, _ in cases], [s for _, s in cases], image_index=[0] * len(cases))
-    for (box, size), o in zip(cases, outs):
-        ref = np.asarray(pil.crop(box).resize(size, Image.BICUBIC))
+    index = [0] * len(cases) + [1]
+    cases.append(((0, 0, 1220, 1220), (224, 224)))
+    outs = proc.resize_u8(devs, [b for b, _ in cases], [s for _, s in cases], image_index=index)
+    for (box, size), i, o in zip(cases, index, outs):
+        ref = np.asarray(pils[i].crop(box).resize(size, Image.BICUBIC))
         assert o.shape == ref.shape and np.array_equal(o.cpu().numpy(), ref), (box, size)
 
 

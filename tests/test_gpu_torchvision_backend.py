@@ -1,6 +1,6 @@
 """GPU (B200, through the C ABI): the torchvision convention of K1 - FusedImageProcessor(backend="torchvision") - is
 bit-identical to the live HF torchvision-backend processor (Qwen2VLImageProcessor, the transformers 5.x default) on the
-test_gpu_k1 geometry list and on every K1 route (tcgen05, IMMA / dp4a, per-tap), with the same launches as the PIL
+test_gpu_k1 geometry list and on every K1 route (tcgen05, dp4a, per-tap), with the same launches as the PIL
 convention; the pre_resize flow and the encoder follow the processor's convention."""
 import numpy as np
 import pytest
@@ -70,13 +70,14 @@ def test_hf_surface_bitexact_vs_live_torchvision_processor(cuda, h, w, box, minp
 
 
 def test_every_k1_route(cuda):
-    """tcgen05 (3 launches: two k1_resample_tc passes + patchify), IMMA / dp4a (an upload 2812 pixels wide: row pitch
-    4 mod 16 and a 6.3x horizontal downscale need 4 B variants x 3 K blocks, more than the tensor-core route holds; at
-    most 31 taps), per-tap (more than 45 taps; and a plain 701-pixel-wide view, row pitch 2103 not a multiple of 4):
+    """tcgen05 (3 launches: two k1_resample_tc passes + patchify), dp4a (an upload 2812 pixels wide: row pitch 4 mod 16
+    and a 6.3x horizontal downscale need 4 B variants x 3 K blocks, more than the tensor-core route holds; at most 31
+    taps; and an upload 1220 pixels wide, row pitch 12 mod 16, at 5.45x on both axes), per-tap (more than 45 taps; and a plain 701-pixel-wide view, row pitch 2103 not a multiple of 4):
     every one bit-identical to the live processor, with the launch count of the PIL convention"""
     from zoomearth_b200 import FusedImageProcessor
     from zoomearth_b200.processor import upload_u8
-    routes = [("tcgen05", _img(1, 1000, 1400), None, 602112, 3), ("IMMA/dp4a", _img(2, 600, 2812), None, 43904, 2),
+    routes = [("tcgen05", _img(1, 1000, 1400), None, 602112, 3), ("dp4a", _img(2, 600, 2812), None, 43904, 2),
+              ("dp4a, pitch 3660", _img(6, 1220, 1220), None, 50176, 2),
               ("per-tap, 109 taps", _img(3, 1500, 1500), None, 3136, 2),
               ("per-tap, pitch 2103", _img(4, 603, 701), (11, 7, 690, 603), 200704, 2)]
     for name, img, box, maxp, launches in routes:

@@ -224,7 +224,7 @@ def test_preprocess_rejects_unknown_kind(lib):
 
 
 def test_tc_route_declines_a_four_variant_pitch_with_three_k_blocks(lib):
-    """the geometry the GPU tests use to reach the IMMA / dp4a kernels: an upload of a 2812-pixel-wide image (row pitch
+    """the geometry the GPU tests use to reach the dp4a kernels: an upload of a 2812-pixel-wide image (row pitch
     4 mod 16, not padded since 2812 is a multiple of 4) downscaled ~7x across: four B variants x three K blocks do not
     fit the tensor-core route's B buffer, 29 taps stay under the dp4a limit of 45"""
     img = _aligned(_img(2, 300, 2812))

@@ -66,7 +66,7 @@ struct PlanDeviceLayout {
   int64_t off_pos = 0;                     // int32 [S][2]: (h, w) rotary ids, window order
   int64_t off_rope = 0;                    // float [max_pos][20][2]: (cos, sin) of pos * inv_freq[j]
   int64_t off_widx = 0;                    // int32 [T]: window position i <-> HF merge-group index
-  int64_t off_win_tiles = 0, off_full_tiles = 0;  // int4 work items (q0, q_len, seg_begin, seg_end)
+  int64_t off_full_tiles = 0;              // int4 work items (q0, q_len, seg_begin, seg_end)
   int64_t off_win_blocks = 0;              // int4 (row0, n_rows, 0, 0): row blocks of whole windows, <= 128 rows (window layers)
   int64_t off_win_bounds = 0;              // int32 [S][2]: (first row, end row) of the window of every patch row
   int32_t max_pos = 0;
@@ -83,8 +83,8 @@ struct zv_plan {
   std::vector<int64_t> window_index, reverse_index;
   std::vector<int32_t> cu_window_raw, cu_window, cu_full;
   std::vector<int32_t> pos_ids;            // [S][2], HF order
-  std::vector<int32_t> win_tiles, full_tiles;   // 4 ints per q tile
+  std::vector<int32_t> full_tiles;              // 4 ints per q tile
   std::vector<int32_t> win_blocks;              // 4 ints per row block of the tcgen05 window kernel
-  int32_t n_win_tiles = 0, n_full_tiles = 0, n_win_blocks = 0;
+  int32_t n_full_tiles = 0, n_win_blocks = 0;
   zv::PlanDeviceLayout dev;
 };

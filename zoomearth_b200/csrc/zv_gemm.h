@@ -110,8 +110,5 @@ int layernorm(const float* x, const float* w, const float* b, void* y, int y_f16
 // patches in HF order (f32 or bf16) -> bf16 in window order (groups of `unit` rows move together)
 int gather_rows(const void* src, int src_dtype, void* dst, int dst_f16, const int32_t* widx, int64_t n_groups, int unit,
                 int cols, void* stream);
-// varlen non-causal attention over q tiles; qkv (S, 3*H) bf16 with rotary already applied
-int attention(const void* qkv, void* out, int heads, int head_dim, const int32_t* tiles_dev, int n_tiles,
-              void* stream, bool full_layer = false, bool f16 = false);
 
 }  // namespace zv

@@ -432,22 +432,17 @@ int zv_plan_create(const zv_cfg* cfg, int32_t n, const int64_t* grid, zv_plan** 
   p->reverse_index.resize(p->T);
   for (int64_t i = 0; i < p->T; ++i) p->reverse_index[p->window_index[i]] = i;
 
-  // attention work items: q tiles of <= 64 rows inside one segment: (q0, q_len, seg_begin, seg_end)
-  auto tiles = [](const std::vector<int32_t>& cu, int32_t bq, std::vector<int32_t>* out_tiles) {
-    for (size_t s = 0; s + 1 < cu.size(); ++s)
-      for (int32_t q0 = cu[s]; q0 < cu[s + 1]; q0 += bq) {
-        out_tiles->push_back(q0);
-        out_tiles->push_back(std::min(bq, cu[s + 1] - q0));
-        out_tiles->push_back(cu[s]);
-        out_tiles->push_back(cu[s + 1]);
-      }
-  };
-  tiles(p->cu_window, 64, &p->win_tiles);      // windows hold <= 64 patches: one 64-row q tile each
-  tiles(p->cu_full, 128, &p->full_tiles);      // whole-image segments: 128-row q tiles (zv_attn.cu, 8 warps)
+  // full layers (tcgen05 kernel): 128-row q tiles inside one whole-image segment: (q0, q_len, seg_begin, seg_end)
+  for (size_t s = 0; s + 1 < p->cu_full.size(); ++s)
+    for (int32_t q0 = p->cu_full[s]; q0 < p->cu_full[s + 1]; q0 += 128) {
+      p->full_tiles.push_back(q0);
+      p->full_tiles.push_back(std::min(128, p->cu_full[s + 1] - q0));
+      p->full_tiles.push_back(p->cu_full[s]);
+      p->full_tiles.push_back(p->cu_full[s + 1]);
+    }
   // window layers (tcgen05 kernel): consecutive whole windows packed greedily into row blocks of <= 128 rows
   build_window_blocks(p->cu_window, 128, &p->win_blocks);
   p->n_win_blocks = (int32_t)(p->win_blocks.size() / 4);
-  p->n_win_tiles = (int32_t)(p->win_tiles.size() / 4);
   p->n_full_tiles = (int32_t)(p->full_tiles.size() / 4);
 
   int32_t max_pos = 0;
@@ -460,7 +455,6 @@ int zv_plan_create(const zv_cfg* cfg, int32_t n, const int64_t* grid, zv_plan** 
   d.off_pos = off; off = align_up(off + (int64_t)S * 2 * sizeof(int32_t), 256);
   d.off_rope = off; off = align_up(off + (int64_t)max_pos * half_rot * 2 * sizeof(float), 256);
   d.off_widx = off; off = align_up(off + p->T * (int64_t)sizeof(int32_t), 256);
-  d.off_win_tiles = off; off = align_up(off + (int64_t)p->win_tiles.size() * sizeof(int32_t), 256);
   d.off_full_tiles = off; off = align_up(off + (int64_t)p->full_tiles.size() * sizeof(int32_t), 256);
   d.off_win_blocks = off; off = align_up(off + (int64_t)p->win_blocks.size() * sizeof(int32_t), 256);
   d.off_win_bounds = off; off = align_up(off + (int64_t)(S + 136) * 2 * sizeof(int32_t), 256);   // + a block of zero padding: the kernel bulk-copies 130 rows from any block start
@@ -496,7 +490,6 @@ void zv::plan_device_image(const zv_plan* p, std::vector<uint8_t>* image) {
       rope[((size_t)ps * half_rot + j) * 2] = (float)std::cos((double)ang);
       rope[((size_t)ps * half_rot + j) * 2 + 1] = (float)std::sin((double)ang);
     }
-  std::memcpy(base + d.off_win_tiles, p->win_tiles.data(), p->win_tiles.size() * sizeof(int32_t));
   std::memcpy(base + d.off_full_tiles, p->full_tiles.data(), p->full_tiles.size() * sizeof(int32_t));
   std::memcpy(base + d.off_win_blocks, p->win_blocks.data(), p->win_blocks.size() * sizeof(int32_t));
   fill_window_bounds(p->cu_window, reinterpret_cast<int32_t*>(base + d.off_win_bounds));

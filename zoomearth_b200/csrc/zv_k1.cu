@@ -72,8 +72,6 @@ struct K1Crop {
   int32_t nwh, nwv;        // words per tap window (fast path), 0 = generic path
   int32_t lh, lw;          // merge-group grid (gh/2, gw/2)
   int32_t fast;            // 1: tmp is row-quad packed (fast path), 0: plain rows
-  int32_t ks_mma;          // horizontal pass on IMMA: 32-byte K steps per 8-column block (1..4), 0 = dp4a kernel
-  int32_t off_mh;          // int32 offset of the IMMA fragment table of the horizontal axis
   int32_t tc;               // 1: both passes on the tensor cores (k1_resample_tc), the kernels below are not used
   uint8_t* dst;            // uint8 output mode (zv_resize_u8): (oh, ow, 3) image, row pitch dst_pitch bytes
   int64_t dst_pitch;
@@ -361,185 +359,6 @@ __global__ void __launch_bounds__(256, NW <= 2 ? 4 : 3) k1_hpass_fast(const K1Cr
   zv::ptx::pdl_trigger();
 }
 
-// Horizontal pass on the tensor cores (mma.sync m16n8k32, u8 x u8 / u8 x s8 -> s32: exact).  dp4a retires 256 int8 MACs per
-// clock per SM, IMMA.16832 2048 (measured, tools/micro/imma_rate.cu), and a Pillow-exact pass is 3 limb products per tap, so
-// the dp4a kernel is bound by its dp4a pipe.  Here D[16 rows x 8 output columns] = A[16 rows x 32 KS source bytes] (one colour
-// plane of the staged strip, row-major: a fragment register is one 32-bit shared load) x B[32 KS x 8] (one limb of the
-// columns' taps, zero outside each column's window; packed per lane by the host, resident in registers for the whole item),
-// one accumulator set per limb.  A warp owns two 8-column blocks of the item's 128-column chunk; strips are 16 rows.  The
-// finished bytes are regrouped across the four lanes of a row group into the row-quad words the vertical pass reads.
-// Fragment table of an axis: per 8-column block 1 + 192 KS ints: first word of the block's source window, then
-// [k step][limb][lane][2] fragment words.
-__device__ __forceinline__ void imma_uu(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void imma_us(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-constexpr int kMRows = 16;          // hpass_mma: source rows per strip (four row quads)
-
-template <int KS>
-__global__ void __launch_bounds__(256, 2) k1_hpass_mma(const K1Crop* __restrict__ crops, const int4* __restrict__ items,
-                                                       int n_items, const int32_t* __restrict__ coef,
-                                                       uint8_t* __restrict__ ws, int plane_pitch) {
-  extern __shared__ uint32_t planes[];            // [16 rows][3 planes][plane_pitch], then raw[2][16][raw_pitch]
-  const int raw_pitch = (plane_pitch * 12 + 32 + 15) & ~15;
-  uint8_t* raw = reinterpret_cast<uint8_t*>(planes + kMRows * 3 * plane_pitch);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int g = lane >> 2, t = lane & 3;
-  constexpr int kStride = 1 + 192 * KS;
-  zv::ptx::pdl_wait();
-
-  for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-    const int4 item = __ldg(items + it);
-    const K1Crop& c = crops[item.x];
-    const uint8_t* __restrict__ src = c.src;
-    const int64_t pitch = c.pitch;
-    const int src_h = c.src_h, ow = c.ow, nq = (c.nrows + 3) >> 2;
-    const int y_base = c.y0 + c.ybox0;
-    const int64_t row_bytes = 3 * (int64_t)c.src_w;
-    const int32_t* __restrict__ lt = coef + c.off_mh;
-    const int xx0 = item.y * kHCols;
-    const int nb0 = xx0 >> 3, nblocks = min(kHCols / 8, (ow - xx0 + 7) >> 3);
-    const int w_first = __ldg(lt + (int64_t)nb0 * kStride);                // window starts are monotone in the block index
-    const int seg_words = min(plane_pitch, __ldg(lt + (int64_t)(nb0 + nblocks - 1) * kStride) + 8 * KS - w_first);
-    const int64_t b0 = 3 * (int64_t)(c.x0 + w_first * 4);                  // first byte of the segment in a row (may be < 0)
-    // this warp's two column blocks: window start and B fragments stay in registers for the whole item
-    int wq0[2];
-    bool blk_ok[2];
-    uint32_t bf[2][KS][3][2];
-#pragma unroll
-    for (int sblk = 0; sblk < 2; ++sblk) {
-      const int nb = warp + 8 * sblk;
-      blk_ok[sblk] = nb < nblocks;
-      const int32_t* __restrict__ e = lt + (int64_t)(nb0 + (blk_ok[sblk] ? nb : 0)) * kStride;
-      wq0[sblk] = __ldg(e) - w_first;
-#pragma unroll
-      for (int ks = 0; ks < KS; ++ks)
-#pragma unroll
-        for (int l = 0; l < 3; ++l) {
-          const int32_t* f = e + 1 + ((ks * 3 + l) * 32 + lane) * 2;       // (the table is only 4-byte aligned)
-          bf[sblk][ks][l][0] = (uint32_t)__ldg(f); bf[sblk][ks][l][1] = (uint32_t)__ldg(f + 1);
-        }
-    }
-    uint32_t* __restrict__ tmp_base = reinterpret_cast<uint32_t*>(ws + c.tmp_off);
-
-    // stage A of strip s: raw bytes of its 16 row segments -> raw[buf] (warp w = rows 2w, 2w + 1); see k1_hpass_fast
-    auto issue = [&](const int strip, const int buf, int (&delta)[2]) {
-#pragma unroll
-      for (int rr = 0; rr < 2; ++rr) {
-        const int rl = 2 * warp + rr;
-        const int y_img = y_base + strip * kMRows + rl;
-        const bool row_ok = y_img >= 0 && y_img < src_h;
-        const uint8_t* rowp = src + (int64_t)(row_ok ? y_img : 0) * pitch;
-        const int dl = (int)((reinterpret_cast<uintptr_t>(rowp) + (uintptr_t)(b0 & 15) + 16) & 15);
-        const int64_t g0 = b0 - dl;
-        const int n_chunks = (dl + seg_words * 12 + 15) >> 4;
-        uint8_t* rraw = raw + (buf * kMRows + rl) * raw_pitch;
-        int ck_lo = 0, ck_hi = 0;
-        if (row_ok) {
-          ck_lo = g0 >= 0 ? 0 : (int)((-g0 + 15) >> 4);
-          ck_hi = (int)min((int64_t)n_chunks, (row_bytes - g0) >> 4);
-          ck_lo = min(ck_lo, n_chunks);
-          ck_hi = max(ck_hi, ck_lo);
-        }
-        const uint32_t dst0 = (uint32_t)__cvta_generic_to_shared(rraw);
-        const uint8_t* src0 = rowp + g0;
-        for (int ck = lane; ck < n_chunks; ck += 32) {
-          if (ck >= ck_lo && ck < ck_hi) {
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst0 + 16 * ck), "l"(src0 + 16 * (int64_t)ck) : "memory");
-          } else {
-            const int64_t o = g0 + 16 * (int64_t)ck;
-            uint32_t wv[4] = {0u, 0u, 0u, 0u};
-            if (row_ok && o + 16 > 0 && o < row_bytes) {
-#pragma unroll
-              for (int k = 0; k < 16; ++k)
-                if (o + k >= 0 && o + k < row_bytes) wv[k >> 2] |= (uint32_t)__ldg(rowp + o + k) << (8 * (k & 3));
-            }
-            *reinterpret_cast<uint4*>(rraw + 16 * ck) = make_uint4(wv[0], wv[1], wv[2], wv[3]);
-          }
-        }
-        delta[rr] = dl;
-      }
-      asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-
-    int delta_cur[2], delta_next[2] = {0, 0};
-    issue(item.z, 0, delta_cur);
-    for (int s = 0; s < item.w; ++s) {
-      const int strip = item.z + s;
-      if (s + 1 < item.w) {
-        issue(strip + 1, (s + 1) & 1, delta_next);
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-      } else {
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-      }
-      __syncthreads();              // every warp is done with the planes of the previous strip; this strip's raw rows landed
-      // ---- stage B: de-interleave this warp's two rows, 4 pixels (12 bytes) per lane step: RGBRGBRGBRGB -> R4 | G4 | B4
-#pragma unroll
-      for (int rr = 0; rr < 2; ++rr) {
-        const int rl = 2 * warp + rr;
-        const uint8_t* rraw = raw + ((s & 1) * kMRows + rl) * raw_pitch;
-        const uint32_t sh = (uint32_t)(delta_cur[rr] & 3) * 8;
-        const uint32_t* wsrc = reinterpret_cast<const uint32_t*>(rraw + (delta_cur[rr] & ~3));
-        uint32_t* p = planes + (rl * 3) * plane_pitch;
-        if (sh == 0) {
-          for (int wq = lane; wq < seg_words; wq += 32) {
-            const uint32_t v0 = wsrc[3 * wq], v1 = wsrc[3 * wq + 1], v2 = wsrc[3 * wq + 2];
-            p[wq] = __byte_perm(__byte_perm(v0, v1, 0x0630), v2, 0x5210);
-            p[plane_pitch + wq] = __byte_perm(__byte_perm(v0, v1, 0x0741), v2, 0x6210);
-            p[2 * plane_pitch + wq] = __byte_perm(__byte_perm(v0, v1, 0x0052), v2, 0x7410);
-          }
-        } else {
-          for (int wq = lane; wq < seg_words; wq += 32) {
-            const uint32_t x0 = wsrc[3 * wq], x1 = wsrc[3 * wq + 1], x2 = wsrc[3 * wq + 2], x3 = wsrc[3 * wq + 3];
-            const uint32_t v0 = __funnelshift_r(x0, x1, sh), v1 = __funnelshift_r(x1, x2, sh), v2 = __funnelshift_r(x2, x3, sh);
-            p[wq] = __byte_perm(__byte_perm(v0, v1, 0x0630), v2, 0x5210);
-            p[plane_pitch + wq] = __byte_perm(__byte_perm(v0, v1, 0x0741), v2, 0x6210);
-            p[2 * plane_pitch + wq] = __byte_perm(__byte_perm(v0, v1, 0x0052), v2, 0x7410);
-          }
-        }
-      }
-      delta_cur[0] = delta_next[0]; delta_cur[1] = delta_next[1];
-      __syncthreads();
-      // ---- compute: warp = two 8-column blocks x 3 channels x 16 rows
-#pragma unroll
-      for (int sblk = 0; sblk < 2; ++sblk) {
-        if (!blk_ok[sblk]) continue;
-        const int col = xx0 + 8 * (warp + 8 * sblk) + 2 * t + ((g & 1));          // this lane's output column after the regroup
-        const int quad = strip * 4 + (g >> 2) + (g & 2);                         // ... and its row quad (g & 2: rows 8-15)
-#pragma unroll
-        for (int ch = 0; ch < 3; ++ch) {
-          int a0c[4] = {0, 0, 0, 0}, a1c[4] = {0, 0, 0, 0}, a2c[4] = {0, 0, 0, 0};
-          const uint32_t* __restrict__ pa = planes + (g * 3 + ch) * plane_pitch + wq0[sblk] + t;
-          const uint32_t* __restrict__ pb = pa + 8 * 3 * plane_pitch;
-#pragma unroll
-          for (int ks = 0; ks < KS; ++ks) {
-            const uint32_t x0 = pa[8 * ks], x1 = pb[8 * ks], x2 = pa[8 * ks + 4], x3 = pb[8 * ks + 4];
-            imma_uu(a0c, x0, x1, x2, x3, bf[sblk][ks][0][0], bf[sblk][ks][0][1]);
-            imma_uu(a1c, x0, x1, x2, x3, bf[sblk][ks][1][0], bf[sblk][ks][1][1]);
-            imma_us(a2c, x0, x1, x2, x3, bf[sblk][ks][2][0], bf[sblk][ks][2][1]);
-          }
-          // bytes of this lane: (row g, col 2t), (row g, col 2t + 1), (row g + 8, col 2t), (row g + 8, col 2t + 1)
-          const uint32_t mine = pack4_sat(finish_raw(a0c[0], a1c[0], a2c[0]), finish_raw(a0c[1], a1c[1], a2c[1]),
-                                          finish_raw(a0c[2], a1c[2], a2c[2]), finish_raw(a0c[3], a1c[3], a2c[3]));
-          // regroup across the four lanes of a row quad (same t, g = 4q .. 4q + 3): lane r = g & 3 collects byte r of each
-          const int base_lane = lane & ~12;
-          const uint32_t y0 = __shfl_sync(0xffffffffu, mine, base_lane), y1 = __shfl_sync(0xffffffffu, mine, base_lane | 4);
-          const uint32_t y2 = __shfl_sync(0xffffffffu, mine, base_lane | 8), y3 = __shfl_sync(0xffffffffu, mine, base_lane | 12);
-          const uint32_t r4 = (uint32_t)(g & 3), sel = r4 | ((4u + r4) << 4);
-          const uint32_t word = __byte_perm(__byte_perm(y0, y1, sel), __byte_perm(y2, y3, sel), 0x5410);   // rows 4q .. 4q + 3
-          if (col < ow && quad < nq) tmp_base[((int64_t)quad * ow + col) * 3 + ch] = word;
-        }
-      }
-    }
-    __syncthreads();                // the next item's first copy may land in raw[0] / its planes pass follows a barrier
-  }
-  zv::ptx::pdl_trigger();
-}
-
 // Vertical pass on dp4a + LUT + patchify.  Item = (crop, merge-group row, first pair, pairs): the 28 output rows' limb
 // tables are parked in shared memory once per item; a unit is two merge groups (28 rows x 56 pixels) whose row quads of
 // the intermediate arrive by 16-byte cp.async (double-buffered), the CTA assembles the two groups' 1176-element patch
@@ -721,17 +540,7 @@ inline int nw_class(int ksize) {                   // words per tap window (<= 3
 }
 
 struct AxisTables { int32_t off_bounds = 0, off_kk = 0, off_limbs = 0, ksize = 0, nw = 0, seg_words = 0, tile_quads = 0;
-                    int32_t off_mma = 0, ks_mma = 0, pitch_mma = 0;
                     int32_t nkb3 = 0, nkb1 = 0; };      // tensor-core route: 128-byte K blocks per 32-byte chunk, 3 channels / 1 channel
-// 32-byte K steps the IMMA horizontal pass needs per 8-column block, from the geometry alone (so that the workspace size
-// does not depend on the tables): 8 neighbouring outputs span at most floor(7 scale) + 2 source samples between their first
-// taps, + ksize taps, + 3 samples of word alignment.  0 = more than 4 steps (the dp4a kernel handles those).
-inline int32_t mma_ksteps(int32_t in_size, int32_t out_size, int32_t ksize) {
-  const double scale = (double)in_size / out_size;
-  const int32_t span = (int32_t)(7.0 * scale) + 2 + ksize + 3;
-  const int32_t ks = (span + 31) / 32;
-  return ks <= 4 ? ks : 0;
-}
 struct Layout {
   int64_t off_desc = 0, off_lut = 0, off_coef = 0, off_lists = 0, off_tmp = 0, bytes = 0;
   int64_t off_tmaps = 0, off_jobs = 0, off_pjobs = 0;     // tensor-core route: 3 tensor maps, 3 RJob and 1 PJob per crop
@@ -749,7 +558,7 @@ struct Layout {
   int64_t item_cap_h = 0, item_cap_v = 0;
 };
 constexpr int kItemsTarget = 148 * 8;        // aim for at least this many work items per launch
-struct AxisCache { std::vector<int32_t> ints; int32_t seg_words = 0, tile_quads = 0, pitch_mma = 0, nkb3 = 0, nkb1 = 0; };
+struct AxisCache { std::vector<int32_t> ints; int32_t seg_words = 0, tile_quads = 0, nkb3 = 0, nkb1 = 0; };
 // K blocks (128 input bytes) the widest 32-output-byte chunk of an axis needs when its samples are `ch` bytes apart
 inline int32_t tc_k_blocks(const zv::AxisCoeffs& ac, int32_t n_out, int32_t ch) {
   int32_t span = 0;
@@ -789,11 +598,7 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
       t.off_bounds = (int32_t)coef_ints;
       t.off_kk = (int32_t)(coef_ints + 2 * (int64_t)key.second);
       t.off_limbs = (int32_t)(coef_ints + 2 * (int64_t)key.second + (int64_t)key.second * t.ksize);
-      t.ks_mma = t.nw > 0 ? mma_ksteps(key.first, key.second, t.ksize) : 0;
-      const int64_t n_blk8 = (key.second + 7) / 8;
-      t.off_mma = (int32_t)(coef_ints + 2 * (int64_t)key.second + (int64_t)key.second * t.ksize + (int64_t)key.second * (1 + 3 * t.nw));
-      const int64_t ints = 2 * (int64_t)key.second + (int64_t)key.second * t.ksize + (int64_t)key.second * (1 + 3 * t.nw) +
-                           (t.ks_mma ? n_blk8 * (1 + 192 * t.ks_mma) : 0);
+      const int64_t ints = 2 * (int64_t)key.second + (int64_t)key.second * t.ksize + (int64_t)key.second * (1 + 3 * t.nw);
       // the tables of an axis depend on (kind, in, out) alone: built once per process and geometry, then copied - a zoom
       // loop asks for the same few sizes over and over and the fp64 tap generation would otherwise pace every small call
       const std::tuple<int32_t, int32_t, int32_t> ckey{kind, key.first, key.second};
@@ -805,7 +610,7 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
       }
       if (fill && hit) {
         L->coef.insert(L->coef.end(), hit->ints.begin(), hit->ints.end());
-        t.seg_words = hit->seg_words; t.tile_quads = hit->tile_quads; t.pitch_mma = hit->pitch_mma;
+        t.seg_words = hit->seg_words; t.tile_quads = hit->tile_quads;
         t.nkb3 = hit->nkb3; t.nkb1 = hit->nkb1;
       } else if (fill) {
         const size_t coef_start = L->coef.size();
@@ -841,56 +646,11 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
         }
         for (int32_t o0 = 0; o0 + 27 < key.second; o0 += 28) t.tile_quads = std::max(t.tile_quads, w0[o0 + 27] + t.nw - w0[o0]);
         if (t.tile_quads == 0) t.tile_quads = 1;            // outputs shorter than 28 (uint8 mode only)
-        if (t.ks_mma) {
-          // IMMA fragment table: per 8-column block the first word of its source window, then, per (k step, limb, lane),
-          // the two B-fragment registers of mma.m16n8k32: b0 = taps k 4t .. 4t + 3, b1 = k 16 + 4t .. of output column g
-          const int32_t KS = t.ks_mma;
-          std::vector<int32_t> bw0((size_t)n_blk8);
-          bool fits = true;
-          for (int64_t nb = 0; nb < n_blk8; ++nb) {
-            const int32_t o0 = (int32_t)(8 * nb), o1 = std::min<int32_t>(key.second, o0 + 8);
-            const int32_t a = ac.bounds[2 * o0] & ~3;
-            bw0[nb] = a >> 2;
-            for (int32_t o = o0; o < o1; ++o) fits = fits && ac.bounds[2 * o] + ac.bounds[2 * o + 1] - a <= 32 * KS;
-          }
-          if (!fits) return zv::fail(ZV_EINVAL, "zv_preprocess: internal: IMMA window bound violated for %d -> %d", key.first, key.second);
-          for (int64_t nb = 0; nb < n_blk8; ++nb) {
-            const int32_t a = bw0[nb] * 4;
-            L->coef.push_back(bw0[nb]);
-            for (int ks = 0; ks < KS; ++ks)
-              for (int limb = 0; limb < 3; ++limb)
-                for (int lane = 0; lane < 32; ++lane) {
-                  const int32_t o = (int32_t)(8 * nb) + (lane >> 2), tq = lane & 3;
-                  for (int half = 0; half < 2; ++half) {
-                    uint32_t word = 0;
-                    for (int b = 0; b < 4; ++b) {
-                      int32_t kv = 0;
-                      if (o < key.second) {
-                        const int32_t tap = a + 32 * ks + 16 * half + 4 * tq + b - ac.bounds[2 * o];
-                        if (tap >= 0 && tap < ac.bounds[2 * o + 1]) kv = ac.kk[(size_t)o * ac.ksize + tap];
-                      }
-                      const uint32_t byte = limb == 0 ? (uint32_t)(kv & 255) : limb == 1 ? (uint32_t)((kv >> 8) & 255)
-                                                                                           : (uint32_t)((kv >> 16) & 255);
-                      word |= byte << (8 * b);
-                    }
-                    L->coef.push_back((int32_t)word);
-                  }
-                }
-          }
-          // widest source span (in words) of a 128-column chunk, as the shared-memory plane pitch: = 4 (mod 8) words, so
-          // that the A-fragment loads of a warp (8 rows x 4 words, rows 3 pitch apart) hit 32 different banks
-          int32_t span = 0;
-          for (int64_t nb = 0; nb < n_blk8; nb += kHCols / 8) {
-            const int64_t last = std::min<int64_t>(n_blk8, nb + kHCols / 8) - 1;
-            span = std::max(span, bw0[last] + 8 * KS - bw0[nb]);
-          }
-          t.pitch_mma = span + ((4 - span % 8) + 8) % 8;
-        }
         t.nkb3 = tc_k_blocks(ac, key.second, 3);
         t.nkb1 = tc_k_blocks(ac, key.second, 1);
         auto entry = std::make_shared<AxisCache>();
         entry->ints.assign(L->coef.begin() + coef_start, L->coef.end());
-        entry->seg_words = t.seg_words; entry->tile_quads = t.tile_quads; entry->pitch_mma = t.pitch_mma;
+        entry->seg_words = t.seg_words; entry->tile_quads = t.tile_quads;
         entry->nkb3 = t.nkb3; entry->nkb1 = t.nkb1;
         std::lock_guard<std::mutex> lock(g_axis_mu);
         if (g_axis_cache.size() >= 512) g_axis_cache.clear();              // bounded: a few hundred KB per entry at most
@@ -939,8 +699,7 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
     const int32_t oh = resized_hw[2 * i], ow = resized_hw[2 * i + 1];
     const int64_t rows = L->nrows[i] + (L->ybox0[i] & 3);
     const int64_t strips = (rows + kHRows - 1) / kHRows, pairs = (ow / 28 + 1) / 2;
-    const int64_t strips16 = (rows + kMRows - 1) / kMRows, per16 = std::max<int64_t>(1, L->strips_per_item / 2);   // IMMA kernel: 16-row strips
-    L->item_cap_h += ((ow + kHCols - 1) / kHCols) * std::max((strips + L->strips_per_item - 1) / L->strips_per_item, (strips16 + per16 - 1) / per16);
+    L->item_cap_h += ((ow + kHCols - 1) / kHCols) * ((strips + L->strips_per_item - 1) / L->strips_per_item);
     L->item_cap_v += u8_out ? (oh + 7) / 8 : (int64_t)(oh / 28) * ((pairs + L->pairs_per_item - 1) / L->pairs_per_item);
   }
   if (L->item_cap_h > INT32_MAX / 8 || L->item_cap_v > INT32_MAX / 8 || L->item_cap_tc > INT32_MAX / 8) return zv::fail(ZV_EINVAL, "zv_preprocess: batch too large for one launch");
@@ -975,15 +734,6 @@ void launch_hfast(int n_items, cudaStream_t s, const K1Crop* d, const int4* item
   if (zv::device_needs_setup(attr, dev)) { cudaFuncSetAttribute(k1_hpass_fast<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); zv::mark_device(attr, dev); }
   zv::launch_pdl(k1_hpass_fast<NW>, dim3((unsigned)persistent_grid(k1_hpass_fast<NW>, smem, n_items)), dim3(256), smem, s, 1,
                  d, items, n_items, coef, ws, seg_words);
-}
-template <int KS>
-void launch_hmma(int n_items, cudaStream_t s, const K1Crop* d, const int4* items, const int32_t* coef, uint8_t* ws, int plane_pitch) {
-  const int smem = kMRows * 3 * plane_pitch * 4 + 2 * kMRows * ((plane_pitch * 12 + 32 + 15) & ~15);
-  static std::atomic<uint64_t> attr{0};
-  const int dev = zv::current_device();
-  if (zv::device_needs_setup(attr, dev)) { cudaFuncSetAttribute(k1_hpass_mma<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024); zv::mark_device(attr, dev); }
-  zv::launch_pdl(k1_hpass_mma<KS>, dim3((unsigned)persistent_grid(k1_hpass_mma<KS>, smem, n_items)), dim3(256), smem, s, 1,
-                 d, items, n_items, coef, ws, plane_pitch);
 }
 inline int vfast_smem(int nw, int tile_quads, int out_bytes) {
   return 2 * tile_quads * 168 * 4 + 2 * 4 * kPatchElems * out_bytes + 768 * 4 + 28 * (1 + 3 * nw) * 4;
@@ -1059,8 +809,8 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
 #else
   const bool generic_only = false;
 #endif
-  std::vector<int32_t> seg_h(n, 0), tq_v(n, 0), pitch_m(n, 0);
-#ifdef ZV_DEBUG_K1_NO_TC                // compile-time debug build: keep every crop on the IMMA / dp4a kernels
+  std::vector<int32_t> seg_h(n, 0), tq_v(n, 0);
+#ifdef ZV_DEBUG_K1_NO_TC                // compile-time debug build: keep every crop on the dp4a / per-tap kernels
   const bool tc_enabled = false;
 #else
   const bool tc_enabled = !generic_only;
@@ -1089,10 +839,6 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
               kHRows * 3 * h.seg_words * 4 + 2 * kHRows * ((h.seg_words * 12 + 32 + 15) & ~15) <= 200 * 1024 &&
               vfast_smem(v.nw, v.tile_quads, 4) <= 200 * 1024) ? 1 : 0;
     c.nwh = c.fast ? h.nw : 0; c.nwv = c.fast ? v.nw : 0;
-    const int mma_smem = kMRows * 3 * h.pitch_mma * 4 + 2 * kMRows * ((h.pitch_mma * 12 + 32 + 15) & ~15);
-    c.ks_mma = (c.fast && h.ks_mma > 0 && mma_smem <= 110 * 1024) ? h.ks_mma : 0;
-    c.off_mh = h.off_mma;
-    pitch_m[i] = h.pitch_mma;
     seg_h[i] = h.seg_words;
     tq_v[i] = v.tile_quads;
     c.ybox0 = L.ybox0[i]; c.nrows = L.nrows[i];
@@ -1115,7 +861,7 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
       c.tc = (tc_enabled && inside && (c.pitch & 3) == 0 && (delta == 0 || 3 * (int64_t)c.src_w + delta <= c.pitch) &&
               4 * c.pitch < (int64_t)1 << 30 && h.nkb3 >= 1 && h.nkb3 <= kTcMaxNkb &&
               h.nkb3 * tc_variants(c.pitch) <= kTcMaxBBlocks && v.nkb1 >= 1 && v.nkb1 <= kTcMaxNkb) ? 1 : 0;
-      if (c.tc) { c.fast = 0; c.nwh = -1; c.nwv = -1; c.ks_mma = 0; ++n_tc; }
+      if (c.tc) { c.fast = 0; c.nwh = -1; c.nwv = -1; ++n_tc; }
     }
     if (c.fast || c.tc) {               // row quads are counted from ybox0 rounded down to 4
       const int32_t al = c.ybox0 & ~3;
@@ -1136,16 +882,13 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
   std::vector<Launch> hl, vl;
   int32_t* lists = reinterpret_cast<int32_t*>(host.data() + L.off_lists);
   int64_t cur = 0;                                    // in ints; items are appended first, so they stay 16-byte aligned
-  // kernel class of a crop's horizontal pass: 100 + KS = IMMA kernel, else the dp4a window class (0 = per-tap kernel)
-  auto hclass = [&](const K1Crop& c) { return c.ks_mma ? 100 + c.ks_mma : c.nwh; };
   auto build = [&](bool vpass, std::vector<Launch>* outl) -> int {
-    for (int nw : {101, 102, 103, 104, 2, 3, 4, 5, 7, 10, 12}) {
-      if (vpass && nw > 100) continue;
+    for (int nw : {2, 3, 4, 5, 7, 10, 12}) {
       Launch l{};
       l.nw = nw; l.list_off = cur;
       for (int32_t i = 0; i < n; ++i) {
         const K1Crop& c = d[i];
-        if ((vpass ? c.nwv : hclass(c)) != nw) continue;
+        if ((vpass ? c.nwv : c.nwh) != nw) continue;
         if (vpass && u8_out) {
           for (int y0 = 0; y0 < c.oh; y0 += 8) {
             lists[cur++] = i; lists[cur++] = y0; lists[cur++] = std::min(8, c.oh - y0); lists[cur++] = 0;
@@ -1157,14 +900,6 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
               lists[cur++] = i; lists[cur++] = my; lists[cur++] = p0; lists[cur++] = std::min(L.pairs_per_item, pairs - p0);
             }
           l.tile_quads = std::max(l.tile_quads, tq_v[i]);
-        } else if (nw > 100) {                      // IMMA kernel: 16-row strips
-          const int strips = (c.nrows + kMRows - 1) / kMRows, chunks = (c.ow + kHCols - 1) / kHCols;
-          const int per = std::max(1, L.strips_per_item / 2);
-          for (int s0 = 0; s0 < strips; s0 += per)
-            for (int ck = 0; ck < chunks; ++ck) {
-              lists[cur++] = i; lists[cur++] = ck; lists[cur++] = s0; lists[cur++] = std::min(per, strips - s0);
-            }
-          l.seg_words = std::max(l.seg_words, pitch_m[i]);
         } else {
           const int strips = (c.nrows + kHRows - 1) / kHRows, chunks = (c.ow + kHCols - 1) / kHCols;
           for (int s0 = 0; s0 < strips; s0 += L.strips_per_item)
@@ -1181,7 +916,7 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
   };
   auto build_generic = [&](bool vpass, std::vector<Launch>* outl) -> int {
     std::vector<int32_t> ids;
-    for (int32_t i = 0; i < n; ++i) if ((vpass ? d[i].nwv : hclass(d[i])) == 0) ids.push_back(i);
+    for (int32_t i = 0; i < n; ++i) if ((vpass ? d[i].nwv : d[i].nwh) == 0) ids.push_back(i);
     if (ids.empty()) return ZV_OK;
     Launch l{};
     l.nw = 0; l.ncls = (int32_t)ids.size();
@@ -1337,10 +1072,6 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
       const int ni = (int)l.count;
       switch (l.nw) {
         case 0: zv::launch_pdl(k1_hpass, dim3((unsigned)l.count), dim3(256), 0, stream, 1, dcrops, list, dlists + l.blk_off, l.ncls, dcoef, ws); break;
-        case 101: launch_hmma<1>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
-        case 102: launch_hmma<2>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
-        case 103: launch_hmma<3>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
-        case 104: launch_hmma<4>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
         case 2: launch_hfast<2>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
         case 3: launch_hfast<3>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;
         case 4: launch_hfast<4>(ni, stream, dcrops, items, dcoef, ws, l.seg_words); break;

@@ -9,7 +9,7 @@
 // produces x also emits x as 16-bit operands (X16) and per-row partial sums of squares (SS), and the consumer GEMM
 // scales its accumulator rows by 1/rms in the epilogue.  No separate norm pass reads X back from HBM.
 //                            QKV = rope((X16 Wqkv'^T) / rms + b)      zv_gemm.cu   EPI_QKV_ROPE
-//                            A = attention(QKV)                       zv_attn.cu / zv_attn_tc.cu
+//                            A = attention(QKV)                       zv_attn_win_tc.cu / zv_attn_tc.cu
 //                            X += A Wo^T + b ; X16, SS                zv_gemm.cu   EPI_RESID
 //                            H = silu((X16 Wg'^T)/rms+b)*((X16 Wu'^T)/rms+b)       EPI_SWIGLU (gate/up rows interleaved)
 //                            X += H Wd^T + b ; X16, SS                             EPI_RESID
@@ -685,18 +685,12 @@ int visual_forward_impl(const zv_cfg* cfg, const void* weights_dev, const zv_pla
   const int32_t* d_pos = reinterpret_cast<const int32_t*>(pd + p->dev.off_pos);
   const float2* d_rope = reinterpret_cast<const float2*>(pd + p->dev.off_rope);
   const int32_t* d_widx = reinterpret_cast<const int32_t*>(pd + p->dev.off_widx);
-  const int32_t* d_win = reinterpret_cast<const int32_t*>(pd + p->dev.off_win_tiles);
   const int32_t* d_full = reinterpret_cast<const int32_t*>(pd + p->dev.off_full_tiles);
   const int32_t* d_wblk = reinterpret_cast<const int32_t*>(pd + p->dev.off_win_blocks);
   const int32_t* d_wbnd = reinterpret_cast<const int32_t*>(pd + p->dev.off_win_bounds);
   float* X = reinterpret_cast<float*>(ws + W.x);
   void* Y = ws + W.y;
   void* BIG = ws + W.big;
-#ifdef ZV_DEBUG_ATTN_LEGACY             // compile-time debug build: mma.sync kernel for the full layers too
-  const bool legacy_full = true;
-#else
-  const bool legacy_full = false;
-#endif
 #define ZV_TRY(expr) do { rc = (expr); if (rc) return rc; } while (0)
 
   // patches -> bf16, window order
@@ -726,8 +720,7 @@ int visual_forward_impl(const zv_cfg* cfg, const void* weights_dev, const zv_pla
       g.bias = reinterpret_cast<const float*>(wb + o.bqkv); g.pos = d_pos; g.rope = d_rope; g.heads = cfg->heads;
       g.row_ln = LNS; g.colsum = reinterpret_cast<const float*>(wb + o.cqkv); g.norm_eps = cfg->eps; g.norm_dim = (int)H;   // norm1
       ZV_TRY(gemm(EPI_QKV_ROPE_LN, g, X16, H, wb + o.wqkv, H, stream));
-      if (!legacy_full) ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
-      else ZV_TRY(attention(BIG, Y, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, true, f16 != 0));
+      ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
       g = GemmArgs{};
       g.op_f16 = f16;
       g.M = (int)S; g.N = (int)H; g.K = (int)H; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
@@ -758,13 +751,10 @@ int visual_forward_impl(const zv_cfg* cfg, const void* weights_dev, const zv_pla
       g.bias = reinterpret_cast<const float*>(wb + o.bqkv); g.pos = d_pos; g.rope = d_rope; g.heads = cfg->heads;
       g.row_ss = SS; g.norm_eps = cfg->eps; g.norm_dim = (int)H;               // norm1 (gain folded into Wqkv)
       ZV_TRY(gemm(EPI_QKV_ROPE, g, X16, H, wb + o.wqkv, H, stream));
-      if (full && !legacy_full) {
+      if (full)
         ZV_TRY(attention_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_full, p->n_full_tiles, stream, f16 != 0));
-      } else if (!full && !legacy_full) {
+      else
         ZV_TRY(attention_win_tc(BIG, Y, S, cfg->heads, (int)(H / cfg->heads), d_wblk, p->n_win_blocks, d_wbnd, stream, f16 != 0));
-      } else {
-        ZV_TRY(attention(BIG, Y, cfg->heads, (int)(H / cfg->heads), full ? d_full : d_win, full ? p->n_full_tiles : p->n_win_tiles, stream, full, f16 != 0));
-      }
       g = GemmArgs{};
       g.op_f16 = f16;
       g.M = (int)S; g.N = (int)H; g.K = (int)H; g.out = X; g.ldo = H; g.out_dtype = ZV_F32;
@@ -828,12 +818,9 @@ int zv_attention(const void* qkv_dev, void* out_dev, int32_t heads, int32_t head
   if (!qkv_dev || !out_dev || !cu_host || n_seg <= 0 || !work_dev) return fail(ZV_EINVAL, "zv_attention: bad argument");
   int rc = check_device("zv_attention");
   if (rc) return rc;
-  std::vector<int32_t> tiles;
   int32_t longest = 0;
   for (int32_t s = 0; s < n_seg; ++s) longest = std::max(longest, cu_host[s + 1] - cu_host[s]);
-  const bool full = longest > 64;                 // same choice the tower makes: 128-row q tiles for long segments
-#ifndef ZV_DEBUG_ATTN_LEGACY
-  if (!full) {
+  if (longest <= 64) {             // same choice the tower makes: the window kernel, else 128-row q tiles for the full one
     // window layers: row blocks + per-row bounds, uploaded into the work buffer, then the tcgen05 window kernel
     std::vector<int32_t> cu(cu_host, cu_host + n_seg + 1), blocks;
     build_window_blocks(cu, 128, &blocks);
@@ -850,27 +837,19 @@ int zv_attention(const void* qkv_dev, void* out_dev, int32_t heads, int32_t head
     return attention_win_tc(qkv_dev, out_dev, S_, heads, head_dim, reinterpret_cast<const int32_t*>(w), (int)(blocks.size() / 4),
                             reinterpret_cast<const int32_t*>(w + off_bounds), stream, dtype == ZV_F16);
   }
-#endif
-  const int32_t bq = full ? 128 : 64;
+  std::vector<int32_t> tiles;
   for (int32_t s = 0; s < n_seg; ++s)
-    for (int32_t q0 = cu_host[s]; q0 < cu_host[s + 1]; q0 += bq) {
-      tiles.push_back(q0); tiles.push_back(std::min(bq, cu_host[s + 1] - q0));
+    for (int32_t q0 = cu_host[s]; q0 < cu_host[s + 1]; q0 += 128) {
+      tiles.push_back(q0); tiles.push_back(std::min(128, cu_host[s + 1] - q0));
       tiles.push_back(cu_host[s]); tiles.push_back(cu_host[s + 1]);
     }
-  int64_t S = cu_host[n_seg];
-#ifdef ZV_DEBUG_ATTN_LEGACY
-  const bool use_tc = false;
-#else
-  const bool use_tc = full;
-#endif
+  const int64_t S = cu_host[n_seg];
   const int64_t need = ((int64_t)tiles.size() * 4 + 255) / 256 * 256;
   if (work_bytes < need) return fail(ZV_ENOMEM, "zv_attention: work buffer %lld B < required %lld B", (long long)work_bytes, (long long)need);
   cudaError_t e = cudaMemcpyAsync(work_dev, tiles.data(), tiles.size() * 4, cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return fail(ZV_ECUDA, "zv_attention: %s", cudaGetErrorString(e));
-  if (use_tc)
-    return attention_tc(qkv_dev, out_dev, S, heads, head_dim, static_cast<const int32_t*>(work_dev), (int)(tiles.size() / 4), stream,
-                        dtype == ZV_F16);
-  return attention(qkv_dev, out_dev, heads, head_dim, static_cast<const int32_t*>(work_dev), (int)(tiles.size() / 4), stream, full, dtype == ZV_F16);
+  return attention_tc(qkv_dev, out_dev, S, heads, head_dim, static_cast<const int32_t*>(work_dev), (int)(tiles.size() / 4), stream,
+                      dtype == ZV_F16);
 }
 
 }  // extern "C"
