@@ -25,7 +25,8 @@
  *                         TorchvisionBackend.rescale_and_normalize (rescale folded into mean and std)
  *   zv_preprocess         infer.py:72-75 (Image.crop) + HF:pil_qwen2_vl.py:143-224 (_preprocess: resize,
  *                         rescale, normalize, patchify) as one fused device pass; by cfg->resample_kind
- *                         HF:models/qwen2_vl/image_processing_qwen2_vl.py (the torchvision backend) instead
+ *                         HF:models/qwen2_vl/image_processing_qwen2_vl.py (the torchvision backend, on the CPU or,
+ *                         kind 2, on a CUDA device) instead
  *   zv_plan_*             HF:models/qwen2_5_vl/modeling_qwen2_5_vl.py:382-409 (rot_pos_emb ids),
  *                         :411-451 (get_window_index), :470-496 (cu_window_seqlens, cu_seqlens)
  *   zv_weights_*          state-dict import of `visual.*` (HF:modeling_qwen2_5_vl.py:345-380 module tree; Qwen2-VL:
@@ -72,8 +73,11 @@ enum { ZV_TOWER_QWEN25 = 0, ZV_TOWER_QWEN2 = 1 };
  * pixels match bit for bit.  ZV_RESAMPLE_PIL: Qwen2VLImageProcessorPil (Pillow bicubic, rescale then normalize).
  * ZV_RESAMPLE_TORCHVISION: Qwen2VLImageProcessor, the transformers 5.x default (torch's uint8 antialiased bicubic:
  * Pillow's windows and weights quantised to int16 at a per-axis precision; normalize with the rescale folded into
- * mean and std, in fp32).  zv_resize_u8 is Pillow-only: it stands for the reference's own resize_image. */
-enum { ZV_RESAMPLE_PIL = 0, ZV_RESAMPLE_TORCHVISION = 1 };
+ * mean and std, in fp32).  ZV_RESAMPLE_TORCHVISION_CUDA: Qwen2VLImageProcessor called with device="cuda" (torch's fp32
+ * antialiased bicubic on a CUDA device: both passes in fp32 with no uint8 rounding between them, then clamp, round half to
+ * even and uint8; the same normalisation as ZV_RESAMPLE_TORCHVISION).  It has no integer taps, so zv_resample_coeffs_ex
+ * rejects it.  zv_resize_u8 is Pillow-only: it stands for the reference's own resize_image. */
+enum { ZV_RESAMPLE_PIL = 0, ZV_RESAMPLE_TORCHVISION = 1, ZV_RESAMPLE_TORCHVISION_CUDA = 2 };
 
 /* Processor + model constants (defaults = Qwen2.5-VL-3B vision config + OPENAI_CLIP statistics). */
 typedef struct zv_cfg {
@@ -97,7 +101,7 @@ typedef struct zv_cfg {
   float   eps;          /* 1e-6 */
   float   reserved_f;
   int32_t tower_kind;   /* ZV_TOWER_QWEN25 (zv_default_cfg) or ZV_TOWER_QWEN2 */
-  int32_t resample_kind; /* ZV_RESAMPLE_PIL (zv_default_cfg) or ZV_RESAMPLE_TORCHVISION */
+  int32_t resample_kind; /* ZV_RESAMPLE_PIL (zv_default_cfg), ZV_RESAMPLE_TORCHVISION or ZV_RESAMPLE_TORCHVISION_CUDA */
 } zv_cfg;
 
 ZV_API const char* zv_version(void);
@@ -249,7 +253,8 @@ ZV_API int64_t zv_last_launch_count(void);
 /* Optional per-kernel-class device timing (CUDA events on the launching stream around every launch of that
  * class).  Classes: 0 k1 hpass, 1 k1 vpass, 2 gemm store, 3 gemm qkv+rope, 4 gemm residual, 5 gemm swiglu,
  * 6 gemm gelu, 7 gemm scatter, 8 attention (window layers), 9 attention (full layers), 10 rmsnorm / layernorm +
- * cast_rows_ss / cast_rows_ln, 11 gather, 12 gemm quickgelu (Qwen2-VL fc1). */
+ * cast_rows_ss / cast_rows_ln, 11 gather, 12 gemm quickgelu (Qwen2-VL fc1), 13 k1 fp32 resample
+ * (ZV_RESAMPLE_TORCHVISION_CUDA; its patchify kernel counts as class 1). */
 ZV_API void zv_timing_enable(int on);
 ZV_API void zv_timing_reset(void);
 ZV_API int zv_timing_read(int kernel_class, double* ms_total, int64_t* count);

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libzoomvit.so")
 ZV_F32, ZV_BF16, ZV_F16 = 0, 1, 2
 ORDER_HF, ORDER_WINDOW = 0, 1
 TOWER_QWEN25, TOWER_QWEN2 = 0, 1
-RESAMPLE_PIL, RESAMPLE_TORCHVISION = 0, 1
+RESAMPLE_PIL, RESAMPLE_TORCHVISION, RESAMPLE_TORCHVISION_CUDA = 0, 1, 2
 ZV_EINVAL, ZV_EINVAL_ASPECT, ZV_EINVAL_BOX, ZV_ENOMEM, ZV_ECUDA, ZV_ENODEV, ZV_EARCH = -1, -2, -3, -4, -5, -6, -7
 
 

@@ -35,7 +35,7 @@ class NvtxRange {
 // Kernel classes for the optional event timing (zv_timing_*): one id per kernel template.
 enum KernelClass { KC_K1_HPASS = 0, KC_K1_VPASS = 1, KC_GEMM_STORE = 2, KC_GEMM_QKV = 3, KC_GEMM_RESID = 4,
                    KC_GEMM_SWIGLU = 5, KC_GEMM_GELU = 6, KC_GEMM_SCATTER = 7, KC_ATTN_WINDOW = 8, KC_ATTN_FULL = 9,
-                   KC_RMSNORM = 10, KC_GATHER = 11, KC_GEMM_QGELU = 12, KC_COUNT = 13 };
+                   KC_RMSNORM = 10, KC_GATHER = 11, KC_GEMM_QGELU = 12, KC_K1_F32 = 13, KC_COUNT = 14 };
 // RAII: records an event pair around the launches issued in its scope when timing is enabled.
 class KernelTimer {
  public:
@@ -50,7 +50,7 @@ class KernelTimer {
 struct AxisCoeffs {
   int32_t in_size = 0, out_size = 0, ksize = 0;
   std::vector<int32_t> bounds;   // [out][2]
-  std::vector<int32_t> kk;       // [out][ksize], 22-bit fixed point
+  std::vector<int32_t> kk;       // [out][ksize], 22-bit fixed point (ZV_RESAMPLE_TORCHVISION_CUDA: fp32 weight bits)
   int32_t precision = 22;        // bits of the taps before they were moved to 22 bits (ZV_RESAMPLE_TORCHVISION: p)
 };
 int32_t resample_ksize(int32_t in_size, int32_t out_size);

@@ -56,8 +56,9 @@ int32_t resample_ksize(int32_t in_size, int32_t out_size) {
 }
 
 int check_resample_kind(int32_t kind, const char* who) {
-  if (kind == ZV_RESAMPLE_PIL || kind == ZV_RESAMPLE_TORCHVISION) return ZV_OK;
-  return fail(ZV_EINVAL, "%s: resample_kind %d (0 ZV_RESAMPLE_PIL, 1 ZV_RESAMPLE_TORCHVISION)", who, kind);
+  if (kind == ZV_RESAMPLE_PIL || kind == ZV_RESAMPLE_TORCHVISION || kind == ZV_RESAMPLE_TORCHVISION_CUDA) return ZV_OK;
+  return fail(ZV_EINVAL, "%s: resample_kind %d (0 ZV_RESAMPLE_PIL, 1 ZV_RESAMPLE_TORCHVISION, 2 ZV_RESAMPLE_TORCHVISION_CUDA)",
+              who, kind);
 }
 
 static void resample_coeffs_pil(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
@@ -127,6 +128,46 @@ static void resample_coeffs_tv(int32_t in_size, int32_t out_size, AxisCoeffs* c)
   }
 }
 
+// torch's fp32 antialiased bicubic on a CUDA device (aten upsample_gen2d_aa_out_frame<float, float, BicubicFilterFunctor>,
+// upsample_antialias::_compute_weights_span / _compute_weights), operation for operation as its sm_100 SASS runs them: the
+// centre scale (i + 0.5) is never rounded on its own - it is folded into FFMAs for the window ends and for xmin - centre -
+// the filter's Horner steps are FFMAs, everything else is a separately rounded fp32 add, multiply or IEEE divide.  The
+// host compiles with -ffp-contract=off, so each std::fma below is the one FFMA and nothing else is fused.  kk holds the
+// weights' fp32 bits.  torch's xsize never exceeds its interp_size = ceilf(support) 2 + 1, which never exceeds Pillow's
+// ksize for the same axis (fl32(in / out) <= k / 2 whenever in / out <= k / 2), so the weights fit Pillow's tap slots.
+static float bicubic_f32(float x) {
+  if (x < 0.0f) x = -x;
+  if (x < 1.0f) return std::fma(x, x * std::fma(x, 1.5f, -2.5f), 1.0f);
+  if (x < 2.0f) return std::fma(x, std::fma(x, x - 5.0f, 8.0f), -4.0f) * -0.5f;
+  return 0.0f;
+}
+
+static void resample_coeffs_f32(int32_t in_size, int32_t out_size, AxisCoeffs* c) {
+  const float scale = (float)in_size / (float)out_size;
+  const float support = scale >= 1.0f ? scale + scale : 2.0f;
+  const float invscale = scale >= 1.0f ? 1.0f / scale : 1.0f;
+  const int32_t ks = c->ksize;
+  std::vector<float> w(ks);
+  for (int32_t xx = 0; xx < out_size; ++xx) {
+    const float ci = (float)xx + 0.5f;
+    const int32_t xmin = std::max((int32_t)(std::fma(ci, scale, -support) + 0.5f), 0);
+    const int32_t xsize = std::min(std::min((int32_t)(std::fma(ci, scale, support) + 0.5f), in_size) - xmin, ks);
+    const float xmin_m_center = std::fma(-ci, scale, (float)xmin);
+    float total = 0.0f;
+    for (int32_t j = 0; j < xsize; ++j) {
+      w[j] = bicubic_f32(((float)j + xmin_m_center + 0.5f) * invscale);
+      total += w[j];
+    }
+    int32_t* k = &c->kk[(size_t)xx * ks];
+    for (int32_t j = 0; j < xsize; ++j) {
+      const float v = total != 0.0f ? w[j] / total : w[j];
+      std::memcpy(&k[j], &v, sizeof(v));
+    }
+    c->bounds[2 * xx] = xmin;
+    c->bounds[2 * xx + 1] = xsize;
+  }
+}
+
 void resample_coeffs(int32_t kind, int32_t in_size, int32_t out_size, AxisCoeffs* c) {
   c->in_size = in_size;
   c->out_size = out_size;
@@ -134,15 +175,21 @@ void resample_coeffs(int32_t kind, int32_t in_size, int32_t out_size, AxisCoeffs
   c->bounds.assign((size_t)out_size * 2, 0);
   c->kk.assign((size_t)out_size * c->ksize, 0);
   c->precision = 22;
-  if (in_size == out_size) {                       // same size: both libraries skip the pass, expressed as one exact tap
+  // same size: both libraries skip the pass, expressed as one exact tap.  torch's fp32 path does run a same-size axis when
+  // the other one is resized, but with scale 1 its taps are (-0, 1, -0, 0) at integer offsets: every output is its
+  // input exactly, the one fp32 tap 1.0f below (up to the sign of a zero, which the final rounding to uint8 drops)
+  if (in_size == out_size) {
+    const float one = 1.0f;
     for (int32_t xx = 0; xx < out_size; ++xx) {
       c->bounds[2 * xx] = xx;
       c->bounds[2 * xx + 1] = 1;
-      c->kk[xx] = 1 << 22;
+      if (kind == ZV_RESAMPLE_TORCHVISION_CUDA) std::memcpy(&c->kk[xx], &one, sizeof(float));
+      else c->kk[xx] = 1 << 22;
     }
     return;
   }
-  if (kind == ZV_RESAMPLE_TORCHVISION) resample_coeffs_tv(in_size, out_size, c);
+  if (kind == ZV_RESAMPLE_TORCHVISION_CUDA) resample_coeffs_f32(in_size, out_size, c);
+  else if (kind == ZV_RESAMPLE_TORCHVISION) resample_coeffs_tv(in_size, out_size, c);
   else resample_coeffs_pil(in_size, out_size, c);
 }
 
@@ -168,7 +215,8 @@ void fill_window_bounds(const std::vector<int32_t>& cu, int32_t* bounds) {
 }
 
 void normalize_lut(const zv_cfg* cfg, float* lut) {
-  if (cfg->resample_kind == ZV_RESAMPLE_TORCHVISION) {
+  // both torchvision conventions: HF builds the same fp32 mean / std tensors and divides with IEEE fp32 on either device
+  if (cfg->resample_kind == ZV_RESAMPLE_TORCHVISION || cfg->resample_kind == ZV_RESAMPLE_TORCHVISION_CUDA) {
     // TorchvisionBackend.rescale_and_normalize: mean' = f32(mean) * f32(1 / rescale), std' likewise, (f32(v) - mean') / std'
     const float inv = (float)(1.0 / cfg->rescale);
     for (int c = 0; c < 3; ++c) {
@@ -347,6 +395,9 @@ int zv_resample_coeffs_ex(int32_t kind, int32_t in_size, int32_t out_size, int32
   if (in_size <= 0 || out_size <= 0 || !bounds || !kk) return fail(ZV_EINVAL, "zv_resample_coeffs_ex: bad argument");
   int rc = check_resample_kind(kind, "zv_resample_coeffs_ex");
   if (rc) return rc;
+  if (kind == ZV_RESAMPLE_TORCHVISION_CUDA)
+    return fail(ZV_EINVAL, "zv_resample_coeffs_ex: resample_kind 2 (ZV_RESAMPLE_TORCHVISION_CUDA) resamples in fp32 and has no "
+                           "integer taps");
   AxisCoeffs c;
   resample_coeffs(kind, in_size, out_size, &c);
   std::memcpy(bounds, c.bounds.data(), c.bounds.size() * sizeof(int32_t));

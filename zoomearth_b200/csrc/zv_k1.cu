@@ -530,6 +530,7 @@ __global__ void __launch_bounds__(256) k1_vpass_u8(const K1Crop* __restrict__ cr
 }
 
 #include "zv_k1_tc.cuh"
+#include "zv_k1_f32.cuh"
 
 // ------------------------------------------------------------------------------------------------ host side
 inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
@@ -618,9 +619,11 @@ int build_layout(int32_t n, const int32_t* crop_box, const int32_t* resized_hw, 
         zv::resample_coeffs(kind, key.first, key.second, &ac);
         L->coef.insert(L->coef.end(), ac.bounds.begin(), ac.bounds.end());
         L->coef.insert(L->coef.end(), ac.kk.begin(), ac.kk.end());
-        // dp4a limb table: the window starts at the first tap rounded down to 4 samples
+        // dp4a limb table: the window starts at the first tap rounded down to 4 samples (left zero for fp32 weights,
+        // which no integer kernel reads)
         std::vector<int32_t> w0(key.second);
-        for (int32_t o = 0; o < key.second; ++o) {
+        if (kind == ZV_RESAMPLE_TORCHVISION_CUDA) L->coef.resize(L->coef.size() + (size_t)key.second * (1 + 3 * t.nw), 0);
+        for (int32_t o = 0; o < key.second && kind != ZV_RESAMPLE_TORCHVISION_CUDA; ++o) {
           const int32_t xmin = ac.bounds[2 * o], cnt = ac.bounds[2 * o + 1];
           const int32_t a = xmin & ~3;
           w0[o] = a >> 2;
@@ -778,6 +781,69 @@ inline bool tc_split_rows(int64_t row0, int64_t nrows, int64_t y_hi, int32_t src
   return *r_b >= (src_h & 3);
 }
 
+// zv_preprocess under ZV_RESAMPLE_TORCHVISION_CUDA: k1_resample_f32 writes each crop's U (the region the tensor-core route
+// uses for it), then k1_patchify_u8 - two launches for any batch.  The layout is the one zv_preprocess_workspace_bytes
+// reports; the fp32 intermediate never leaves shared memory.
+int k1_run_f32(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* src_dev, const int32_t* src_hw,
+               const int64_t* src_pitch, const int32_t* crop_box, const int32_t* resized_hw, const int64_t* row_off,
+               void* out_dev, int32_t out_dtype, int32_t row_order, const Layout& L, void* workspace_dev, cudaStream_t stream) {
+  std::vector<uint8_t> host((size_t)L.off_tmp, 0);
+  K1Crop* d = reinterpret_cast<K1Crop*>(host.data() + L.off_desc);
+  PJob* pjobs = reinterpret_cast<PJob*>(host.data() + L.off_pjobs);
+  int32_t* blk0 = reinterpret_cast<int32_t*>(host.data() + L.off_lists);
+  uint8_t* ws = static_cast<uint8_t*>(workspace_dev);
+  int64_t row = 0, tiles = 0, groups = 0;
+  for (int32_t i = 0; i < n; ++i) {
+    K1Crop& c = d[i];
+    c.src = src_dev[i]; c.pitch = src_pitch[i];
+    c.src_h = src_hw[2 * i]; c.src_w = src_hw[2 * i + 1];
+    c.x0 = crop_box[4 * i]; c.y0 = crop_box[4 * i + 1];
+    c.cw = crop_box[4 * i + 2] - c.x0; c.ch = crop_box[4 * i + 3] - c.y0;
+    c.oh = resized_hw[2 * i]; c.ow = resized_hw[2 * i + 1];
+    if (!c.src || c.pitch < 3 * (int64_t)c.src_w) return zv::fail(ZV_EINVAL, "%s: image %d has a null pointer or short pitch", who, i);
+    const AxisTables& h = L.axis.at({c.cw, c.ow});
+    const AxisTables& v = L.axis.at({c.ch, c.oh});
+    c.ksh = h.ksize; c.ksv = v.ksize;
+    c.off_bh = h.off_bounds; c.off_kh = h.off_kk; c.off_bv = v.off_bounds; c.off_kv = v.off_kk;
+    c.dst = ws + L.off_tmp + L.u_off[i]; c.dst_pitch = 3 * (int64_t)c.ow;
+    c.lh = c.oh / 28; c.lw = c.ow / 28;
+    c.out_row0 = row_off ? row_off[i] : row;
+    row += (int64_t)(c.oh / 14) * (c.ow / 14);
+    blk0[i] = (int32_t)tiles;
+    tiles += f32_tiles(c.oh, c.ow);
+    PJob& pj = pjobs[i];
+    pj.u = c.dst; pj.u_pitch = c.dst_pitch; pj.out_row0 = c.out_row0; pj.lh = c.lh; pj.lw = c.lw; pj.blk0 = (int32_t)groups;
+    groups += (int64_t)c.lh * c.lw;
+    if (tiles > INT32_MAX || groups > INT32_MAX) return zv::fail(ZV_EINVAL, "zv_preprocess: batch too large for one launch");
+  }
+  zv::normalize_lut(cfg, reinterpret_cast<float*>(host.data() + L.off_lut));
+  std::memcpy(host.data() + L.off_coef, L.coef.data(), L.coef.size() * sizeof(int32_t));
+  cudaError_t e = cudaMemcpyAsync(ws, host.data(), host.size(), cudaMemcpyHostToDevice, stream);
+  if (e != cudaSuccess) return zv::fail(ZV_ECUDA, "%s: table upload: %s", who, cudaGetErrorString(e));
+  const K1Crop* dcrops = reinterpret_cast<const K1Crop*>(ws + L.off_desc);
+  const int32_t* dcoef = reinterpret_cast<const int32_t*>(ws + L.off_coef);
+  const float* dlut = reinterpret_cast<const float*>(ws + L.off_lut);
+  const PJob* dpj = reinterpret_cast<const PJob*>(ws + L.off_pjobs);
+  {
+    zv::KernelTimer timer(zv::KC_K1_F32, stream);
+    zv::launch_pdl(k1_resample_f32, dim3((unsigned)tiles), dim3(kF32Threads), 0, stream, 1, dcrops,
+                   reinterpret_cast<const int32_t*>(ws + L.off_lists), (int)n, dcoef);
+    zv::count_launch();
+  }
+  {
+    zv::KernelTimer timer(zv::KC_K1_VPASS, stream);
+    const int wsz = cfg->window / cfg->merge / cfg->patch;
+    const unsigned blocks = (unsigned)std::min<int64_t>(groups, (int64_t)zv::num_sms() * 8);
+    if (out_dtype == ZV_BF16) zv::launch_pdl(k1_patchify_u8<__nv_bfloat16>, dim3(blocks), dim3(256), 0, stream, 1, dpj, (int)n, (int)groups, dlut, static_cast<__nv_bfloat16*>(out_dev), (int)row_order, wsz);
+    else if (out_dtype == ZV_F16) zv::launch_pdl(k1_patchify_u8<__half>, dim3(blocks), dim3(256), 0, stream, 1, dpj, (int)n, (int)groups, dlut, static_cast<__half*>(out_dev), (int)row_order, wsz);
+    else zv::launch_pdl(k1_patchify_u8<float>, dim3(blocks), dim3(256), 0, stream, 1, dpj, (int)n, (int)groups, dlut, static_cast<float*>(out_dev), (int)row_order, wsz);
+    zv::count_launch();
+  }
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return zv::fail(ZV_ECUDA, "%s: launch: %s", who, cudaGetErrorString(e));
+  return ZV_OK;
+}
+
 // Both device entry points: the two resample passes over n crops.  u8_dst == nullptr: patches (LUT + patchify) into out_dev;
 // else plain uint8 images into u8_dst[i] (row pitch u8_pitch[i]).
 int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* src_dev, const int32_t* src_hw,
@@ -800,6 +866,11 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
   if (rc) return rc;
   if (workspace_bytes < L.bytes)
     return zv::fail(ZV_ENOMEM, "%s: workspace %lld B < required %lld B", who, (long long)workspace_bytes, (long long)L.bytes);
+  if (kind == ZV_RESAMPLE_TORCHVISION_CUDA) {           // never the integer kernels; no crop takes the tensor-core route
+    if (emulate_tc) { std::fill(emulate_tc, emulate_tc + n, 0); return ZV_OK; }
+    return k1_run_f32(who, cfg, n, src_dev, src_hw, src_pitch, crop_box, resized_hw, row_off, out_dev, out_dtype, row_order, L,
+                      workspace_dev, stream);
+  }
 
   // host image of [descriptors | LUT | coefficient tables | launch lists]
   std::vector<uint8_t> host((size_t)L.off_tmp, 0);

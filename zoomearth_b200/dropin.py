@@ -7,7 +7,8 @@ path is ``model.visual`` on transformers 4.49 (what the reference pins) and ``mo
 
 ``image_backend`` picks the HF image-processor backend whose pixels the fused processor reproduces.  On transformers
 5.x ``AutoProcessor`` hands Qwen2-VL / Qwen2.5-VL the torchvision backend whenever torchvision is installed, so a 5.x
-user who wants the model to keep seeing the same ``pixel_values`` passes ``image_backend="match"``.
+user who wants the model to keep seeing the same ``pixel_values`` passes ``image_backend="match"``; a torchvision
+processor built with ``device="cuda"`` resamples in fp32 on the GPU, which "match" maps to "torchvision_cuda".
 """
 import torch
 
@@ -34,8 +35,9 @@ def _bicubic(resample):
 
 def _image_backend(old, image_backend):
     """The FusedImageProcessor backend for ``install(..., image_backend=...)`` replacing the image processor ``old``."""
-    if image_backend not in ("pil", "torchvision", "match"):
-        raise ValueError(f"image_backend must be 'pil', 'torchvision' or 'match', got {image_backend!r}")
+    if image_backend not in ("pil", "torchvision", "torchvision_cuda", "match"):
+        raise ValueError("image_backend must be 'pil', 'torchvision', 'torchvision_cuda' or 'match', "
+                         f"got {image_backend!r}")
     if image_backend == "pil":
         return "pil"
     backend = image_backend
@@ -45,12 +47,14 @@ def _image_backend(old, image_backend):
         except ImportError:
             PilBackend = TorchvisionBackend = ()
         if TorchvisionBackend and isinstance(old, TorchvisionBackend):
-            backend = "torchvision"
+            device = getattr(old, "device", None)
+            backend = "torchvision_cuda" if device is not None and torch.device(device).type == "cuda" else "torchvision"
         elif PilBackend and isinstance(old, PilBackend):
             backend = "pil"
         else:
             raise ValueError(f"image_backend='match': cannot tell which backend {type(old).__name__} resamples with "
-                             "(known: transformers 5.x TorchvisionBackend / PilBackend); pass 'pil' or 'torchvision'")
+                             "(known: transformers 5.x TorchvisionBackend / PilBackend); pass 'pil', 'torchvision' or "
+                             "'torchvision_cuda'")
     resample = getattr(old, "resample", None)
     if not _bicubic(resample):
         raise NotImplementedError(f"{type(old).__name__} resamples with {resample!r}; the fused processor reproduces "
@@ -60,10 +64,11 @@ def _image_backend(old, image_backend):
 
 def install(model=None, processor=None, device=None, dtype=None, image_backend="pil"):
     """Returns (fused_visual or None, fused_image_processor or None).  ``image_backend``: "pil" (the default) matches
-    HF's PIL backend; "torchvision" matches HF's torchvision backend; "match" reads which of the two
-    ``processor.image_processor`` is (a transformers 5.x ``TorchvisionBackend`` or ``PilBackend`` instance, anything else
-    is a ValueError).  Under "torchvision" / "match" a replaced processor that does not resample bicubic raises
-    NotImplementedError."""
+    HF's PIL backend; "torchvision" matches HF's torchvision backend on the CPU; "torchvision_cuda" matches it with
+    ``device="cuda"``; "match" reads which of these ``processor.image_processor`` is (a transformers 5.x
+    ``TorchvisionBackend`` - "torchvision_cuda" when its ``device`` is a CUDA device - or ``PilBackend`` instance,
+    anything else is a ValueError).  Under any choice but "pil" a replaced processor that does not resample bicubic
+    raises NotImplementedError."""
     fv = fp = None
     backend = _image_backend(processor.image_processor, image_backend) if processor is not None else None
     if model is not None:

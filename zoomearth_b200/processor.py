@@ -9,7 +9,10 @@ Pillow bicubic -> rescale -> normalize -> patchify); results are bit-identical t
 ``backend="torchvision"`` they are bit-identical to HF's torchvision backend instead
 (``models/qwen2_vl/image_processing_qwen2_vl.py``, what ``AutoImageProcessor`` returns on transformers 5.x when
 torchvision is installed): torch's uint8 antialiased bicubic and the fp32 fused rescale + normalize.  The device
-kernels are the same; only the coefficient tables and the normalisation LUT differ.
+kernels are the same; only the coefficient tables and the normalisation LUT differ.  With
+``backend="torchvision_cuda"`` they are bit-identical to that processor called with ``device="cuda"``: torch's fp32
+antialiased bicubic as a CUDA device runs it (no uint8 rounding between the two passes), which K1 runs as its own
+fp32 kernel.
 
 Also the crop-aware entry ``preprocess_crops`` used by the zoom fast path: the source image stays resident on
 the GPU as uint8 and every zoom step reads its crop box straight out of it (``Image.crop`` semantics of
@@ -102,7 +105,16 @@ def _to_u8_hwc(image):
     return image.contiguous()
 
 
-BACKENDS = {"pil": _lib.RESAMPLE_PIL, "torchvision": _lib.RESAMPLE_TORCHVISION}
+BACKENDS = {"pil": _lib.RESAMPLE_PIL, "torchvision": _lib.RESAMPLE_TORCHVISION,
+            "torchvision_cuda": _lib.RESAMPLE_TORCHVISION_CUDA}
+
+
+def _backend_for_device(backend, device):
+    """HF's torchvision processor resamples on ``device`` when a call passes one: a CUDA device runs torch's fp32 path,
+    the CPU its uint8 path.  The PIL backend has no such argument."""
+    if device is None or backend == "pil":
+        return backend
+    return "torchvision_cuda" if torch.device(device).type == "cuda" else "torchvision"
 
 
 class FusedImageProcessor:
@@ -112,9 +124,12 @@ class FusedImageProcessor:
     def __init__(self, min_pixels=None, max_pixels=None, size=None, patch_size=14, temporal_patch_size=2,
                  merge_size=2, image_mean=None, image_std=None, rescale_factor=1 / 255, device=None,
                  output_device="cpu", backend="pil", **unused):
-        """``backend``: which HF image-processor backend the pixels match bit for bit - "pil" (Qwen2VLImageProcessorPil)
-        or "torchvision" (Qwen2VLImageProcessor).  It applies to ``preprocess`` / ``__call__`` and ``preprocess_crops``;
-        ``resize_u8`` / ``cut_resize`` are the reference's own Pillow ``resize_image`` under either."""
+        """``backend``: which HF image-processor backend the pixels match bit for bit - "pil" (Qwen2VLImageProcessorPil),
+        "torchvision" (Qwen2VLImageProcessor on the CPU) or "torchvision_cuda" (Qwen2VLImageProcessor with
+        ``device="cuda"``).  It applies to ``preprocess`` / ``__call__`` and ``preprocess_crops``; ``resize_u8`` /
+        ``cut_resize`` are the reference's own Pillow ``resize_image`` under any.  As in HF, a ``device=`` passed to
+        ``preprocess`` / ``__call__`` picks the torchvision convention of that call (a CUDA device "torchvision_cuda",
+        the CPU "torchvision"); under "pil" it is ignored."""
         if backend not in BACKENDS:
             raise ValueError(f"backend must be one of {sorted(BACKENDS)}, got {backend!r}")
         self.backend = backend
@@ -153,12 +168,12 @@ class FusedImageProcessor:
     def max_pixels(self, v):
         self.size["longest_edge"] = v
 
-    def _cfg(self, min_pixels=None, max_pixels=None):
+    def _cfg(self, min_pixels=None, max_pixels=None, backend=None):
         return _lib.default_cfg(patch=self.patch_size, merge=self.merge_size, temporal=self.temporal_patch_size,
                                 min_pixels=int(min_pixels if min_pixels is not None else self.min_pixels),
                                 max_pixels=int(max_pixels if max_pixels is not None else self.max_pixels),
                                 rescale=float(self.rescale_factor), mean=self.image_mean, std=self.image_std,
-                                resample_kind=BACKENDS[self.backend])
+                                resample_kind=BACKENDS[backend or self.backend])
 
     def _device(self):
         if self.device is None:
@@ -181,12 +196,14 @@ class FusedImageProcessor:
 
     # ---- device path
     def preprocess_crops(self, images_dev, boxes=None, out_dtype=torch.float32, window_order=False,
-                         min_pixels=None, max_pixels=None, image_index=None, apply_cut_image=False, out=None):
+                         min_pixels=None, max_pixels=None, image_index=None, apply_cut_image=False, out=None,
+                         backend=None):
         """images_dev: list of (H, W, 3) uint8 CUDA tensors.  boxes: (n, 4) crop boxes (x0, y0, x1, y1) in image
         pixels, or None for the whole image; ``image_index[i]`` says which image crop i reads (default i).
         ``apply_cut_image`` first maps each box through the reference's cut_image() rule (min 512 px).
+        ``backend`` overrides the processor's backend for this call.
         Returns (patches (S, 1176) out_dtype on the GPU, image_grid_thw (n, 3) int64 CPU tensor, crop boxes)."""
-        cfg = self._cfg(min_pixels, max_pixels)
+        cfg = self._cfg(min_pixels, max_pixels, backend)
         device = images_dev[0].device
         if device.type != "cuda":
             raise RuntimeError("preprocess_crops takes CUDA tensors; there is no CPU path")
@@ -200,7 +217,7 @@ class FusedImageProcessor:
         else:
             # final crop boxes, PIL.Image.crop semantics: int(round(v)) with Python's round-half-even
             bx = np.rint(np.asarray(boxes, np.float64)).astype(np.int64).reshape(n, 4)
-            cfg0 = self._cfg(min_pixels, max_pixels)
+            cfg0 = self._cfg(min_pixels, max_pixels, backend)
             cfg0.min_size = -1                     # boxes are final crop boxes: no cut_image rule
             crop, rhw, grid = geometry.geometry(cfg0, img_hw, bx.astype(np.float64))
         S = int((grid[:, 1] * grid[:, 2]).sum())
@@ -321,7 +338,7 @@ class FusedImageProcessor:
 
     # ---- HF surface
     def preprocess(self, images, videos=None, return_tensors=None, min_pixels=None, max_pixels=None, size=None,
-                   do_resize=None, do_rescale=None, do_normalize=None, **unused):
+                   do_resize=None, do_rescale=None, do_normalize=None, device=None, **unused):
         if videos is not None:
             raise NotImplementedError("FusedImageProcessor covers the image branch only (the reference uses no video)")
         for name, flag in (("do_resize", do_resize), ("do_rescale", do_rescale), ("do_normalize", do_normalize)):
@@ -330,12 +347,13 @@ class FusedImageProcessor:
         if size is not None:
             min_pixels = size.get("shortest_edge", min_pixels)
             max_pixels = size.get("longest_edge", max_pixels)
-        device = self._device()
+        backend = _backend_for_device(self.backend, device)     # the HF kwarg picks the convention, not where K1 runs
         imgs = [_to_u8_hwc(i) for i in _flatten(images)]
         if not imgs:
             raise ValueError("no images given")
-        dev_imgs = [upload_u8(t, device) for t in imgs]
-        pv, grid, _ = self.preprocess_crops(dev_imgs, None, torch.float32, False, min_pixels, max_pixels)
+        dev_imgs = [upload_u8(t, self._device()) for t in imgs]
+        pv, grid, _ = self.preprocess_crops(dev_imgs, None, torch.float32, False, min_pixels, max_pixels,
+                                            backend=backend)
         if self.output_device == "cpu":
             pv = pv.cpu()
         data = {"pixel_values": pv, "image_grid_thw": grid}
