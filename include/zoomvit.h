@@ -27,6 +27,8 @@
  *                         rescale, normalize, patchify) as one fused device pass; by cfg->resample_kind
  *                         HF:models/qwen2_vl/image_processing_qwen2_vl.py (the torchvision backend, on the CPU or,
  *                         kind 2, on a CUDA device) instead
+ *   zv_preprocess_video   HF:models/qwen2_vl/video_processing_qwen2_vl.py (Qwen2VLVideoProcessor, torchvision resize on the
+ *                         CPU or a CUDA device) as one device pass over all frames of a batch of videos
  *   zv_plan_*             HF:models/qwen2_5_vl/modeling_qwen2_5_vl.py:382-409 (rot_pos_emb ids),
  *                         :411-451 (get_window_index), :470-496 (cu_window_seqlens, cu_seqlens)
  *   zv_weights_*          state-dict import of `visual.*` (HF:modeling_qwen2_5_vl.py:345-380 module tree; Qwen2-VL:
@@ -148,6 +150,21 @@ ZV_API int zv_preprocess(const zv_cfg* cfg, int32_t n, const uint8_t* const* src
                          const int64_t* src_pitch, const int32_t* crop_box, const int32_t* resized_hw,
                          const int64_t* row_off, void* out_dev, int32_t out_dtype, int32_t row_order,
                          void* workspace_dev, int64_t workspace_bytes, void* stream);
+
+/* Video frames -> patches (HF:models/qwen2_vl/video_processing_qwen2_vl.py Qwen2VLVideoProcessor._preprocess: resize,
+ * fused rescale + normalize, last-frame repeat to an even count, patchify with temporal patches of two frames).
+ * frames_per_video[v] = T_v >= 1; frame f (all videos' frames back to back) is frame_dev[f], (H, W, 3) uint8 of size
+ * frame_hw[f] = (h, w) with row pitch frame_pitch[f] bytes; video v's frames are resized whole to resized_hw[v] (multiples of
+ * 28).  Video v writes ceil(T_v / 2) * gh * gw patch rows (1176 elements of out_dtype), videos back to back; temporal slot
+ * tp of frame group t holds frame min(2 t + tp, T_v - 1).  row_order: HF order, or the tower's window order inside every
+ * frame group.  cfg->resample_kind must be ZV_RESAMPLE_TORCHVISION (HF's video processor on the CPU) or
+ * ZV_RESAMPLE_TORCHVISION_CUDA (on a CUDA device); ZV_RESAMPLE_PIL is ZV_EINVAL, HF has no PIL video backend. */
+ZV_API int64_t zv_preprocess_video_workspace_bytes(int32_t n_videos, const int32_t* frames_per_video, const int32_t* frame_hw,
+                                                   const int32_t* resized_hw);
+ZV_API int zv_preprocess_video(const zv_cfg* cfg, int32_t n_videos, const int32_t* frames_per_video,
+                               const uint8_t* const* frame_dev, const int32_t* frame_hw, const int64_t* frame_pitch,
+                               const int32_t* resized_hw, void* out_dev, int32_t out_dtype, int32_t row_order,
+                               void* workspace_dev, int64_t workspace_bytes, void* stream);
 
 /* Device form of the reference's resize_image(cut_image(...)): crop i = PIL.Image.crop(crop_box[i]) of image i (zero
  * fill outside the image), resized with Pillow-exact bicubic to out_hw[i] = (h, w) and written as a plain (h, w, 3) uint8

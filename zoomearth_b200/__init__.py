@@ -12,6 +12,9 @@ def __getattr__(name):            # torch-dependent pieces are imported lazily
     if name == "FusedImageProcessor":
         from .processor import FusedImageProcessor
         return FusedImageProcessor
+    if name == "FusedVideoProcessor":
+        from .video import FusedVideoProcessor
+        return FusedVideoProcessor
     if name == "FusedVisual":
         from .visual import FusedVisual
         return FusedVisual

@@ -60,6 +60,9 @@ _PROTOS = {
     "zv_preprocess_workspace_bytes": (C.c_int64, [C.c_int32, C.c_void_p, C.c_void_p]),
     "zv_preprocess": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "zv_preprocess_video_workspace_bytes": (C.c_int64, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zv_preprocess_video": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "zv_debug_k1_tc_host": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "zv_plan_create": (C.c_int, [_P(ZvCfg), C.c_int32, C.c_void_p, _P(C.c_void_p)]),

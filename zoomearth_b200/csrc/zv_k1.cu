@@ -531,6 +531,7 @@ __global__ void __launch_bounds__(256) k1_vpass_u8(const K1Crop* __restrict__ cr
 
 #include "zv_k1_tc.cuh"
 #include "zv_k1_f32.cuh"
+#include "zv_k1_video.cuh"
 
 // ------------------------------------------------------------------------------------------------ host side
 inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
@@ -783,10 +784,12 @@ inline bool tc_split_rows(int64_t row0, int64_t nrows, int64_t y_hi, int32_t src
 
 // zv_preprocess under ZV_RESAMPLE_TORCHVISION_CUDA: k1_resample_f32 writes each crop's U (the region the tensor-core route
 // uses for it), then k1_patchify_u8 - two launches for any batch.  The layout is the one zv_preprocess_workspace_bytes
-// reports; the fp32 intermediate never leaves shared memory.
+// reports; the fp32 intermediate never leaves shared memory.  u8_dst != nullptr (the video path): U goes to u8_dst[i] (row
+// pitch u8_pitch[i]) and nothing is patchified - one launch.
 int k1_run_f32(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* src_dev, const int32_t* src_hw,
                const int64_t* src_pitch, const int32_t* crop_box, const int32_t* resized_hw, const int64_t* row_off,
-               void* out_dev, int32_t out_dtype, int32_t row_order, const Layout& L, void* workspace_dev, cudaStream_t stream) {
+               void* out_dev, int32_t out_dtype, int32_t row_order, uint8_t* const* u8_dst, const int64_t* u8_pitch,
+               const Layout& L, void* workspace_dev, cudaStream_t stream) {
   std::vector<uint8_t> host((size_t)L.off_tmp, 0);
   K1Crop* d = reinterpret_cast<K1Crop*>(host.data() + L.off_desc);
   PJob* pjobs = reinterpret_cast<PJob*>(host.data() + L.off_pjobs);
@@ -805,7 +808,8 @@ int k1_run_f32(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* con
     const AxisTables& v = L.axis.at({c.ch, c.oh});
     c.ksh = h.ksize; c.ksv = v.ksize;
     c.off_bh = h.off_bounds; c.off_kh = h.off_kk; c.off_bv = v.off_bounds; c.off_kv = v.off_kk;
-    c.dst = ws + L.off_tmp + L.u_off[i]; c.dst_pitch = 3 * (int64_t)c.ow;
+    c.dst = u8_dst ? u8_dst[i] : ws + L.off_tmp + L.u_off[i]; c.dst_pitch = u8_dst ? u8_pitch[i] : 3 * (int64_t)c.ow;
+    if (!c.dst || c.dst_pitch < 3 * (int64_t)c.ow) return zv::fail(ZV_EINVAL, "%s: output %d has a null pointer or short pitch", who, i);
     c.lh = c.oh / 28; c.lw = c.ow / 28;
     c.out_row0 = row_off ? row_off[i] : row;
     row += (int64_t)(c.oh / 14) * (c.ow / 14);
@@ -830,7 +834,7 @@ int k1_run_f32(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* con
                    reinterpret_cast<const int32_t*>(ws + L.off_lists), (int)n, dcoef);
     zv::count_launch();
   }
-  {
+  if (!u8_dst) {
     zv::KernelTimer timer(zv::KC_K1_VPASS, stream);
     const int wsz = cfg->window / cfg->merge / cfg->patch;
     const unsigned blocks = (unsigned)std::min<int64_t>(groups, (int64_t)zv::num_sms() * 8);
@@ -868,8 +872,8 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
     return zv::fail(ZV_ENOMEM, "%s: workspace %lld B < required %lld B", who, (long long)workspace_bytes, (long long)L.bytes);
   if (kind == ZV_RESAMPLE_TORCHVISION_CUDA) {           // never the integer kernels; no crop takes the tensor-core route
     if (emulate_tc) { std::fill(emulate_tc, emulate_tc + n, 0); return ZV_OK; }
-    return k1_run_f32(who, cfg, n, src_dev, src_hw, src_pitch, crop_box, resized_hw, row_off, out_dev, out_dtype, row_order, L,
-                      workspace_dev, stream);
+    return k1_run_f32(who, cfg, n, src_dev, src_hw, src_pitch, crop_box, resized_hw, row_off, out_dev, out_dtype, row_order,
+                      u8_dst, u8_pitch, L, workspace_dev, stream);
   }
 
   // host image of [descriptors | LUT | coefficient tables | launch lists]
@@ -1221,9 +1225,130 @@ int k1_run(const char* who, const zv_cfg* cfg, int32_t n, const uint8_t* const* 
   return ZV_OK;
 }
 
+// zv_preprocess_video's workspace: [video jobs | LUT | the uint8 frames U, 256-byte aligned each | K1's uint8-mode
+// workspace for all frames].  Every frame is a whole-frame crop resized to its video's size.
+struct VideoLayout {
+  int64_t off_lut = 0, off_u = 0, off_k1 = 0, bytes = 0;
+  int32_t total = 0;
+  std::vector<int64_t> u_off;                // per frame, relative to off_u
+  std::vector<int32_t> crop, rhw;            // per frame: (0, 0, w, h) and its video's (oh, ow)
+};
+int video_layout(const char* who, int32_t n_videos, const int32_t* frames, const int32_t* frame_hw, const int32_t* resized_hw,
+                 VideoLayout* V) {
+  int64_t total = 0;
+  for (int32_t v = 0; v < n_videos; ++v) {
+    if (frames[v] <= 0) return zv::fail(ZV_EINVAL, "%s: video %d has %d frames", who, v, frames[v]);
+    const int32_t oh = resized_hw[2 * v], ow = resized_hw[2 * v + 1];
+    if (oh <= 0 || ow <= 0 || oh % 28 || ow % 28)
+      return zv::fail(ZV_EINVAL, "%s: video %d resized to %dx%d (need >0 and multiples of 28)", who, v, ow, oh);
+    total += frames[v];
+    if (total > INT32_MAX / 4) return zv::fail(ZV_EINVAL, "%s: too many frames", who);
+  }
+  V->total = (int32_t)total;
+  V->u_off.resize(total); V->crop.resize(4 * total); V->rhw.resize(2 * total);
+  int64_t f = 0, u = 0;
+  for (int32_t v = 0; v < n_videos; ++v) {
+    const int32_t oh = resized_hw[2 * v], ow = resized_hw[2 * v + 1];
+    for (int32_t k = 0; k < frames[v]; ++k, ++f) {
+      V->crop[4 * f] = 0; V->crop[4 * f + 1] = 0; V->crop[4 * f + 2] = frame_hw[2 * f + 1]; V->crop[4 * f + 3] = frame_hw[2 * f];
+      V->rhw[2 * f] = oh; V->rhw[2 * f + 1] = ow;
+      V->u_off[f] = u;
+      u += align_up((int64_t)oh * ow * 3, 256);
+    }
+  }
+  Layout L;
+  int rc = build_layout(V->total, V->crop.data(), V->rhw.data(), &L, false, true);
+  if (rc) return rc;
+  int64_t off = align_up((int64_t)n_videos * (int64_t)sizeof(VJob), 256);
+  V->off_lut = off; off = align_up(off + 768 * (int64_t)sizeof(float), 256);
+  V->off_u = off; off += u;
+  V->off_k1 = off; off += L.bytes;
+  V->bytes = off;
+  return ZV_OK;
+}
+
 }  // namespace
 
 extern "C" {
+
+int64_t zv_preprocess_video_workspace_bytes(int32_t n_videos, const int32_t* frames_per_video, const int32_t* frame_hw,
+                                            const int32_t* resized_hw) {
+  if (n_videos <= 0 || !frames_per_video || !frame_hw || !resized_hw)
+    return zv::fail(ZV_EINVAL, "zv_preprocess_video_workspace_bytes: bad argument");
+  VideoLayout V;
+  int rc = video_layout("zv_preprocess_video_workspace_bytes", n_videos, frames_per_video, frame_hw, resized_hw, &V);
+  return rc ? rc : V.bytes;
+}
+
+int zv_preprocess_video(const zv_cfg* cfg, int32_t n_videos, const int32_t* frames_per_video, const uint8_t* const* frame_dev,
+                        const int32_t* frame_hw, const int64_t* frame_pitch, const int32_t* resized_hw, void* out_dev,
+                        int32_t out_dtype, int32_t row_order, void* workspace_dev, int64_t workspace_bytes, void* stream_) {
+  const char* who = "zv_preprocess_video";
+  zv::reset_launch_count();
+  zv::NvtxRange nvtx_k1("zv:K1 video frames->patches");
+  if (!cfg || n_videos <= 0 || !frames_per_video || !frame_dev || !frame_hw || !frame_pitch || !resized_hw || !out_dev ||
+      !workspace_dev)
+    return zv::fail(ZV_EINVAL, "%s: null argument", who);
+  if (cfg->patch != 14 || cfg->merge != 2 || cfg->temporal != 2)
+    return zv::fail(ZV_EINVAL, "%s: only patch=14, merge=2, temporal=2 is built", who);
+  if (out_dtype != ZV_F32 && out_dtype != ZV_BF16 && out_dtype != ZV_F16) return zv::fail(ZV_EINVAL, "%s: bad out_dtype", who);
+  if (row_order != ZV_ORDER_HF && row_order != ZV_ORDER_WINDOW) return zv::fail(ZV_EINVAL, "%s: bad row_order", who);
+  int rc = zv::check_resample_kind(cfg->resample_kind, who);
+  if (rc) return rc;
+  if (cfg->resample_kind == ZV_RESAMPLE_PIL)
+    return zv::fail(ZV_EINVAL, "%s: resample_kind 0 (ZV_RESAMPLE_PIL): HF's video processor has no PIL backend; it resamples "
+                               "with torchvision (kind 1 on the CPU, kind 2 on a CUDA device)", who);
+  VideoLayout V;
+  rc = video_layout(who, n_videos, frames_per_video, frame_hw, resized_hw, &V);
+  if (rc) return rc;
+  if (workspace_bytes < V.bytes)
+    return zv::fail(ZV_ENOMEM, "%s: workspace %lld B < required %lld B", who, (long long)workspace_bytes, (long long)V.bytes);
+  uint8_t* ws = static_cast<uint8_t*>(workspace_dev);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  std::vector<uint8_t*> u8_dst(V.total);
+  std::vector<int64_t> u8_pitch(V.total);
+  for (int32_t f = 0; f < V.total; ++f) {
+    u8_dst[f] = ws + V.off_u + V.u_off[f];
+    u8_pitch[f] = 3 * (int64_t)V.rhw[2 * f + 1];
+  }
+  // every frame of every video in one pass of the image routes, uint8 out (launch counts accumulate from here)
+  rc = k1_run(who, cfg, V.total, frame_dev, frame_hw, frame_pitch, V.crop.data(), V.rhw.data(), nullptr, nullptr, 0, 0,
+              u8_dst.data(), u8_pitch.data(), ws + V.off_k1, workspace_bytes - V.off_k1, stream);
+  if (rc) return rc;
+  std::vector<uint8_t> host((size_t)V.off_u, 0);
+  VJob* jobs = reinterpret_cast<VJob*>(host.data());
+  int64_t row = 0, groups = 0, f0 = 0;
+  for (int32_t v = 0; v < n_videos; ++v) {
+    VJob& j = jobs[v];
+    const int32_t oh = resized_hw[2 * v], ow = resized_hw[2 * v + 1], gt = (frames_per_video[v] + 1) / 2;
+    j.u = u8_dst[f0];
+    j.frame_bytes = frames_per_video[v] > 1 ? V.u_off[f0 + 1] - V.u_off[f0] : 0;
+    j.out_row0 = row;
+    j.lh = oh / 28; j.lw = ow / 28; j.frames = frames_per_video[v]; j.blk0 = (int32_t)groups;
+    row += (int64_t)gt * (oh / 14) * (ow / 14);
+    groups += (int64_t)gt * j.lh * j.lw;
+    f0 += frames_per_video[v];
+    if (groups > INT32_MAX) return zv::fail(ZV_EINVAL, "%s: batch too large for one launch", who);
+  }
+  zv::normalize_lut(cfg, reinterpret_cast<float*>(host.data() + V.off_lut));
+  cudaError_t e = cudaMemcpyAsync(ws, host.data(), host.size(), cudaMemcpyHostToDevice, stream);
+  if (e != cudaSuccess) return zv::fail(ZV_ECUDA, "%s: table upload: %s", who, cudaGetErrorString(e));
+  {
+    zv::KernelTimer timer(zv::KC_K1_VPASS, stream);
+    const VJob* dj = reinterpret_cast<const VJob*>(ws);
+    const float* dlut = reinterpret_cast<const float*>(ws + V.off_lut);
+    const int wsz = cfg->window / cfg->merge / cfg->patch;
+    const unsigned blocks = (unsigned)std::min<int64_t>(groups, (int64_t)zv::num_sms() * 8);
+    if (out_dtype == ZV_BF16) zv::launch_pdl(k1_patchify_video<__nv_bfloat16>, dim3(blocks), dim3(256), 0, stream, 1, dj, (int)n_videos, (int)groups, dlut, static_cast<__nv_bfloat16*>(out_dev), (int)row_order, wsz);
+    else if (out_dtype == ZV_F16) zv::launch_pdl(k1_patchify_video<__half>, dim3(blocks), dim3(256), 0, stream, 1, dj, (int)n_videos, (int)groups, dlut, static_cast<__half*>(out_dev), (int)row_order, wsz);
+    else zv::launch_pdl(k1_patchify_video<float>, dim3(blocks), dim3(256), 0, stream, 1, dj, (int)n_videos, (int)groups, dlut, static_cast<float*>(out_dev), (int)row_order, wsz);
+    zv::count_launch();
+  }
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return zv::fail(ZV_ECUDA, "%s: launch: %s", who, cudaGetErrorString(e));
+  return ZV_OK;
+}
+
 
 int64_t zv_preprocess_workspace_bytes(int32_t n, const int32_t* crop_box, const int32_t* resized_hw) {
   if (n <= 0 || !crop_box || !resized_hw) return zv::fail(ZV_EINVAL, "zv_preprocess_workspace_bytes: bad argument");

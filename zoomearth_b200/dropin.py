@@ -13,6 +13,7 @@ processor built with ``device="cuda"`` resamples in fp32 on the GPU, which "matc
 import torch
 
 from .processor import FusedImageProcessor
+from .video import FusedVideoProcessor
 from .visual import FusedVisual
 
 
@@ -62,15 +63,34 @@ def _image_backend(old, image_backend):
     return backend
 
 
-def install(model=None, processor=None, device=None, dtype=None, image_backend="pil"):
+def _video_backend(old, video_backend):
+    """The FusedVideoProcessor backend for ``install(..., video_backend=...)`` replacing the video processor ``old``: the
+    rules of ``_image_backend``, without "pil" (HF's video processor always resamples with torchvision)."""
+    if video_backend not in ("torchvision", "torchvision_cuda", "match"):
+        raise ValueError("video_backend must be None, 'torchvision', 'torchvision_cuda' or 'match' (HF has no PIL video "
+                         f"backend), got {video_backend!r}")
+    if old is None:
+        raise ValueError("video_backend given but the processor has no video_processor to replace")
+    backend = _image_backend(old, video_backend)
+    if backend == "pil":
+        raise ValueError(f"video_backend='match': {type(old).__name__} is a PIL backend; HF's video processor has none")
+    return backend
+
+
+def install(model=None, processor=None, device=None, dtype=None, image_backend="pil", video_backend=None):
     """Returns (fused_visual or None, fused_image_processor or None).  ``image_backend``: "pil" (the default) matches
     HF's PIL backend; "torchvision" matches HF's torchvision backend on the CPU; "torchvision_cuda" matches it with
     ``device="cuda"``; "match" reads which of these ``processor.image_processor`` is (a transformers 5.x
     ``TorchvisionBackend`` - "torchvision_cuda" when its ``device`` is a CUDA device - or ``PilBackend`` instance,
     anything else is a ValueError).  Under any choice but "pil" a replaced processor that does not resample bicubic
-    raises NotImplementedError."""
+    raises NotImplementedError.  ``video_backend``: None (the default) leaves ``processor.video_processor`` as it is;
+    "torchvision", "torchvision_cuda" or "match" replace it with a FusedVideoProcessor under the same rules (HF's
+    ``Qwen2VLVideoProcessor`` is a ``TorchvisionBackend``).  The fused tower serves video grids either way."""
     fv = fp = None
     backend = _image_backend(processor.image_processor, image_backend) if processor is not None else None
+    vbackend = None
+    if processor is not None and video_backend is not None:
+        vbackend = _video_backend(getattr(processor, "video_processor", None), video_backend)
     if model is not None:
         owner = _find_visual(model)
         hf_visual = owner.visual
@@ -90,4 +110,14 @@ def install(model=None, processor=None, device=None, dtype=None, image_backend="
                                  image_mean=getattr(old, "image_mean", None), image_std=getattr(old, "image_std", None),
                                  device=device, backend=backend)
         processor.image_processor = fp
+        if vbackend is not None:
+            old = processor.video_processor
+            processor.video_processor = FusedVideoProcessor(
+                size=dict(getattr(old, "size", None) or {}) or None, patch_size=getattr(old, "patch_size", 14),
+                temporal_patch_size=getattr(old, "temporal_patch_size", 2), merge_size=getattr(old, "merge_size", 2),
+                image_mean=getattr(old, "image_mean", None), image_std=getattr(old, "image_std", None),
+                rescale_factor=getattr(old, "rescale_factor", 1 / 255), device=device, backend=vbackend,
+                do_sample_frames=bool(getattr(old, "do_sample_frames", False)), num_frames=getattr(old, "num_frames", None),
+                fps=getattr(old, "fps", None), min_frames=getattr(old, "min_frames", 4),
+                max_frames=getattr(old, "max_frames", 768), return_metadata=bool(getattr(old, "return_metadata", False)))
     return fv, fp

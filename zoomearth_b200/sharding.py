@@ -13,11 +13,13 @@ import torch.distributed as dist
 
 def crop_cost(grid_thw, full_layers=4):
     """FLOP estimate per crop (SURVEY 8e) of a 32-block tower: linear + full attention + window attention.
-    ``full_layers``: blocks with full attention (4 in Qwen2.5-VL, all 32 in Qwen2-VL); the rest attend in windows."""
+    ``full_layers``: blocks with full attention (4 in Qwen2.5-VL, all 32 in Qwen2-VL); the rest attend in windows.
+    Full attention never crosses a frame group of a video (HF cu_seqlens = repeat_interleave(h w, t)): t (h w)^2."""
     g = np.asarray(grid_thw, dtype=np.float64).reshape(-1, 3)
-    S = g[:, 0] * g[:, 1] * g[:, 2]
+    HW = g[:, 1] * g[:, 2]
+    S = g[:, 0] * HW
     T = S / 4
-    return 5.125e9 * T + full_layers * 4 * S * S * 1280 + (32 - full_layers) * 4 * 64 * S * 1280
+    return 5.125e9 * T + full_layers * 4 * S * HW * 1280 + (32 - full_layers) * 4 * 64 * S * 1280
 
 
 def partition(costs, world_size):

@@ -94,6 +94,26 @@ class ZoomEncoder:
             return emb, grid, crop, pv
         return emb, grid, crop
 
+    @torch.no_grad()
+    def encode_video(self, videos_dev, min_pixels=None, max_pixels=None, backend="torchvision_cuda", use_graph=False,
+                     return_patches=False):
+        """The device-resident video path: videos_dev, a list of (T, H, W, 3) uint8 CUDA tensors, -> window-ordered
+        16-bit patches (``zv_preprocess_video``, every frame in one call) -> the tower.  ``backend`` picks the resampling
+        HF's video processor would run: "torchvision_cuda" (frames on a CUDA device, the default here) or "torchvision"
+        (the CPU).  ``min_pixels`` / ``max_pixels`` default to the video processor's (128 / 768 x 28^2).
+        Returns (embeddings (T, out_hidden) in HF order, video_grid_thw (n, 3))."""
+        if not hasattr(self, "video_processor"):
+            from .video import FusedVideoProcessor
+            self.video_processor = FusedVideoProcessor(device=self.visual.device, backend=backend)
+        vp = self.video_processor
+        pv, grid = vp.preprocess_videos(videos_dev, out_dtype=self.visual.operand_dtype, window_order=True,
+                                        min_pixels=min_pixels, max_pixels=max_pixels, backend=backend)
+        emb = self.visual(pv, grid, window_order=True, use_graph=use_graph)
+        self.last_launches = vp.last_launches + self.visual.last_launches
+        if return_patches:
+            return emb, grid, pv
+        return emb, grid
+
     def micro_batches(self, images_dev, boxes, image_index=None, max_patches=400_000, apply_cut_image=True):
         """Splits a ragged crop list into consecutive micro-batches of at most ``max_patches`` patches (a crop larger
         than the budget is a batch of its own), so the tower's workspace stays bounded whatever the batch
