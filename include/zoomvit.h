@@ -40,6 +40,7 @@
  *   zv_rope_index         reference .../open_r1/model/modeling_qwen2_vl.py:967-1114 (get_rope_index; by flag the
  *                         transformers 5.x variant HF:modeling_qwen2_5_vl.py:1024-1135)
  *   zv_placeholder_rows   the row list behind masked_scatter (HF:modeling_qwen2_5_vl.py:1179-1218)
+ *   zv_rope_index_dev, zv_placeholder_rows_dev   the same two on the device, stream-ordered and graph-capturable
  */
 #ifndef ZOOMVIT_H_
 #define ZOOMVIT_H_
@@ -264,7 +265,42 @@ ZV_API int zv_rope_index(const int64_t* input_ids, const int64_t* attention_mask
 ZV_API int64_t zv_placeholder_rows(const int64_t* input_ids, int64_t n_tokens, int64_t image_token_id,
                                    int64_t* rows_out, int64_t rows_cap);
 
-/* Number of kernels the last zv_preprocess / zv_visual_forward call on this thread launched. */
+/* ---------------------------------------------------------------- LM hand-off, device side */
+/* The two functions above as kernels on `stream`: device pointers in and out, no host synchronisation, no allocation, so
+ * that they can be captured in one CUDA graph with zv_visual_forward_into.  Results are bit-identical to the host
+ * functions.  A condition on which zv_rope_index fails is recorded in `status` (int64 [4] on the device) instead:
+ *   status[0] = ZV_HANDOFF_* check (0 = none), status[1] = sample, status[2..3] = details (below);
+ * the error recorded is the one the host function reports: the lowest sample, then the host's check order.  On such an
+ * error the positions are unspecified; nothing is written outside the caller's buffers.  Argument errors the host can
+ * see (null pointers, batch / seq_len / merge <= 0, a workspace smaller than zv_handoff_workspace_bytes) return ZV_EINVAL
+ * before any device work.  One workspace serves both functions for the same (batch, seq_len) on one stream. */
+enum {
+  ZV_HANDOFF_OK = 0,
+  ZV_HANDOFF_VIDEO = 1,             /* a vision start followed by a video placeholder */
+  ZV_HANDOFF_TRAILING_VSTART = 2,   /* the sample's last admitted token is a vision start */
+  ZV_HANDOFF_FEW_PLACEHOLDERS = 3,  /* fewer image placeholders than images */
+  ZV_HANDOFF_GRID_ROWS = 4,         /* image_grid_thw has too few rows; status[2] = n_images */
+  ZV_HANDOFF_EMPTY_GRID = 5,        /* status[2] = the image (grid row) with t, h / merge or w / merge <= 0 */
+  ZV_HANDOFF_COUNT = 6,             /* status[2] positions for status[3] tokens */
+  ZV_HANDOFF_MASKED = 7,            /* every token of the sample is masked */
+  ZV_HANDOFF_ROWS_COUNT = 8         /* zv_placeholder_rows_dev: status[2] placeholders for status[3] = rows_cap rows */
+};
+ZV_API int64_t zv_handoff_workspace_bytes(int32_t batch, int32_t seq_len);
+/* input_ids, attention_mask (may be NULL): [batch][seq_len] int64; image_grid_thw: [n_images][3] int64 (NULL = text
+ * only); position_ids [3][batch][seq_len], deltas [batch]; all on the device.  2 kernel launches (1 without a grid). */
+ZV_API int zv_rope_index_dev(const int64_t* input_ids, const int64_t* attention_mask, int32_t batch, int32_t seq_len,
+                             const int64_t* image_grid_thw, int32_t n_images, int64_t image_token_id,
+                             int64_t video_token_id, int64_t vision_start_token_id, int32_t merge, int32_t hf5_semantics,
+                             int64_t* position_ids, int64_t* deltas, int64_t* status, void* workspace_dev,
+                             int64_t workspace_bytes, void* stream);
+/* rows_out [rows_cap]: the flattened indices of input_ids == image_token_id in order (masked_scatter order), -1 in every
+ * slot at or beyond their count; status[2] = the count, status[0] = ZV_HANDOFF_ROWS_COUNT when it is not rows_cap.
+ * The workspace needs zv_handoff_workspace_bytes of any (batch, seq_len) with batch * seq_len >= n_tokens.  2 launches. */
+ZV_API int zv_placeholder_rows_dev(const int64_t* input_ids, int64_t n_tokens, int64_t image_token_id, int64_t* rows_out,
+                                   int64_t rows_cap, int64_t* status, void* workspace_dev, int64_t workspace_bytes,
+                                   void* stream);
+
+/* Number of kernels the last zv_preprocess / zv_visual_forward / hand-off device call on this thread launched. */
 ZV_API int64_t zv_last_launch_count(void);
 
 /* Optional per-kernel-class device timing (CUDA events on the launching stream around every launch of that

@@ -27,7 +27,7 @@ def __getattr__(name):            # torch-dependent pieces are imported lazily
     if name == "install":
         from .dropin import install
         return install
-    if name in ("get_rope_index", "embed_images", "placeholder_rows"):
+    if name in ("get_rope_index", "embed_images", "placeholder_rows", "DeviceHandoff"):
         from . import handoff
         return getattr(handoff, name)
     if name == "Plan":

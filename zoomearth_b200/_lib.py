@@ -93,6 +93,12 @@ _PROTOS = {
     "zv_rope_index": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_int64,
                                 C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "zv_placeholder_rows": (C.c_int64, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64]),
+    "zv_handoff_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32]),
+    "zv_rope_index_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_int64,
+                                    C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                    C.c_void_p]),
+    "zv_placeholder_rows_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                          C.c_int64, C.c_void_p]),
     "zv_last_launch_count": (C.c_int64, []),
     "zv_timing_enable": (None, [C.c_int]),
     "zv_timing_reset": (None, []),

@@ -16,7 +16,7 @@ INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libzoomvit.so")
 OBJ_DIR = os.path.join(HERE, "_build")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-SOURCES = ["zv_host.cpp", "zv_handoff.cpp", "zv_k1.cu", "zv_gemm.cu", "zv_attn_tc.cu", "zv_attn_win_tc.cu", "zv_tower.cu", "zv_timing.cu"]
+SOURCES = ["zv_host.cpp", "zv_handoff.cpp", "zv_handoff.cu", "zv_k1.cu", "zv_gemm.cu", "zv_attn_tc.cu", "zv_attn_win_tc.cu", "zv_tower.cu", "zv_timing.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-I", INCLUDE, "-I", CSRC,
           "-Xcompiler", "-fPIC,-fvisibility=hidden,-ffp-contract=off,-Wall,-Wno-unused-function"]
@@ -36,7 +36,7 @@ def needs_build():
 
 
 def _compile(src):
-    obj = os.path.join(OBJ_DIR, src.rsplit(".", 1)[0] + ".o")
+    obj = os.path.join(OBJ_DIR, src + ".o")          # zv_handoff.cpp and zv_handoff.cu both build
     cmd = [NVCC] + ARCH + COMMON + ["-x", "cu", "-c", os.path.join(CSRC, src), "-o", obj]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode:
